@@ -10,6 +10,11 @@ One JSON line on stdout (rank 0).  `value` times rs_transcribe_device with the w
 resident in HBM; `e2e` times rs_transcribe_batch (the model.transcribe seam of the C ABI) with
 pinned HOST buffers, H2D and D2H inside the timed region.  Weights are seeded random weights of the
 619 M architecture (no checkpoint is reachable offline), data is synthetic; both are stated.
+
+    python bench.py --steps K --dump-outputs DIR    # also write the last timed step's outputs as DIR/*.npy
+
+The inputs depend on the arguments only, so two builds run with the same arguments can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -146,6 +151,27 @@ def python_api_multi_gpu_rtfx(cfg, n_gpus: int, n_clips: int, seconds: float):
             "what": "one process, load_model(devices=[0..N-1]) + transcribe_batch(model, audios): numpy clips in, TranscribeResult out"}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, tokens: torch.Tensor, frames: torch.Tensor, n_tok: torch.Tensor):
+    """Write what rs_transcribe_device returned (tokens / frames int32 [B, U], n_tok int32 [B]) as float32 .npy files.
+    Entries past a clip's token count are unspecified by the C ABI and written as -1.  When the arrays exceed
+    DUMP_BYTES, a fixed seeded sample of clips is written, with their batch indices in clips.npy."""
+    B, U = tokens.shape
+    clips = np.arange(B)
+    per_clip = (2 * U + 2) * 4
+    if B * per_clip > DUMP_BYTES:
+        clips = np.sort(np.random.default_rng(0).choice(B, DUMP_BYTES // per_clip, replace=False))
+    n = n_tok.numpy()[clips]
+    valid = np.arange(U)[None, :] < np.minimum(n, U)[:, None]
+    arrays = {"tokens": np.where(valid, tokens.numpy()[clips], -1), "frames": np.where(valid, frames.numpy()[clips], -1),
+              "n_tokens": n, "clips": clips}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float32))
+
+
 def make_batch(n_clips: int, seconds: float, rank: int):
     from reazonspeech_b200.synth import synth_clip
     L = int(seconds * 16000) + 2 * PAD
@@ -279,7 +305,13 @@ def main():
     ap.add_argument("--seconds", type=float, default=NOMINAL_SECONDS)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip python_api / decode_sensitivity / config2 (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's tokens / frames / token counts (rank 0) "
+                                                           "as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -341,6 +373,8 @@ def main():
     ms_step = ms_total / args.steps
     value = world * B * args.seconds / (ms_step / 1e3)
     n_tok = out_dev[2].cpu()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out_dev[0].cpu(), out_dev[1].cpu(), n_tok)
 
     # ---------------- end-to-end through the host-buffer C-ABI call (`e2e`)
     for _ in range(2):
