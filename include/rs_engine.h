@@ -175,16 +175,20 @@ int rs_layernorm(rs_engine* e, const float* x, const float* gamma, const float* 
                  void* stream);
 /* Counters: kernels launched by this engine since creation (bench.py's gpu_launches). */
 int64_t rs_launch_count(const rs_engine* e);
-/* Per-stage device time of the last rs_transcribe_* call when timing was enabled. */
+/* Per-stage device time of the last rs_transcribe_* call when timing was enabled: ms[0..4] = log-mel, subsampling,
+ * conformer layers, f32->bf16 + joint.enc GEMM, greedy decode (ms[5..7] are zero).  Every entry point records the
+ * stage marks.  The log-mel stage ends at the log-mel of the last utterance chunk, so for rs_transcribe_batch /
+ * _pcm16 with chunked copies (B >= 16) it includes the host-to-device copies and the first subsampling conv of the
+ * chunks before the last one, which overlap it. */
 int rs_enable_stage_timing(rs_engine* e, int on);
 int rs_stage_times_ms(const rs_engine* e, float* ms /*[8]*/);
+int rs_debug_decode_cycles(rs_engine* e, int B, int L_max, int U_max, int64_t* out8);   /* profiling aid, see engine.cu */
+int rs_debug_attention_cycles(rs_engine* e, int64_t* out16);   /* clock64 stamps of one CTA of the last attention launch */
+int rs_debug_gemm_cycles(rs_engine* e, int64_t* out64);        /* clock64 timeline of the last 2-CTA GEMM launch: first / last cluster x 32 stamps (gemm_tcgen05.cu) */
 /* Per-launch CUDA-event timing of the tcgen05 GEMM (the dominant kernel): while enabled every GEMM
  * launch is bracketed by two events on its stream.  rs_gemm_timing() synchronises, returns the summed
  * device time, the summed algorithmic FLOPs (2*M*N*K) and the launch count since it was enabled or
  * last read, and resets the accumulators. */
-int rs_debug_decode_cycles(rs_engine* e, int B, int L_max, int U_max, int64_t* out8);   /* profiling aid, see engine.cu */
-int rs_debug_attention_cycles(rs_engine* e, int64_t* out16);   /* clock64 stamps of one CTA of the last attention launch */
-int rs_debug_gemm_cycles(rs_engine* e, int64_t* out64);        /* clock64 timeline of the last 2-CTA GEMM launch: first / last cluster x 32 stamps (gemm_tcgen05.cu) */
 int rs_enable_gemm_timing(rs_engine* e, int on);
 int rs_gemm_timing(rs_engine* e, double* ms, double* flops, int64_t* launches);
 /* Per-kernel CUDA-event timing of EVERY launch inside the real pipeline (warm caches, back-to-back launches, unlike

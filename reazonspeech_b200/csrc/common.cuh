@@ -194,14 +194,6 @@ __device__ __forceinline__ void tma_load_2d_2sm(uint32_t smem_dst, const void* d
       ::"r"(smem_dst), "l"(desc), "r"(bar & kPeerBitMask), "r"(c0), "r"(c1)
       : "memory");
 }
-// Multicast form: the tile lands at the same CTA-relative offset in every CTA of `mask`, and each destination credits
-// the same-offset barrier of ITS pair leader (CUTLASS SM100_TMA_2SM_LOAD_MULTICAST).
-__device__ __forceinline__ void tma_load_2d_2sm_mc(uint32_t smem_dst, const void* desc, int c0, int c1, uint32_t bar, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%4, %5}], [%2], %3;"
-      ::"r"(smem_dst), "l"(desc), "r"(bar & kPeerBitMask), "h"(mask), "r"(c0), "r"(c1)
-      : "memory");
-}
 // mbarrier.arrive on the same-offset barrier of CTA `cta` of the cluster.
 __device__ __forceinline__ void mbar_arrive_remote(uint32_t bar, uint32_t cta) {
   asm volatile(
@@ -225,11 +217,6 @@ __device__ __forceinline__ void umma_commit_2sm(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                ::"r"(bar), "h"(static_cast<uint16_t>(3)) : "memory");
 }
-// commit -> arrive on the same-offset barrier of every CTA in `mask`
-__device__ __forceinline__ void umma_commit_2sm_mask(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"(mask) : "memory");
-}
 __device__ __forceinline__ void umma_bf16_ss_2sm(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
@@ -237,13 +224,6 @@ __device__ __forceinline__ void umma_bf16_ss_2sm(uint32_t tmem_d, uint64_t desc_
       "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
       ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
-}
-
-// ---------------------------------------------------------------- vector global access
-__device__ __forceinline__ uint4 ldg_nc_v4(const void* p) {
-  uint4 r;
-  asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-  return r;
 }
 
 }  // namespace rs

@@ -76,12 +76,6 @@ __device__ __forceinline__ void sp_grid_barrier(unsigned int* counters, unsigned
   __syncthreads();
 }
 
-__device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
 __device__ __forceinline__ void mma_f16_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
   asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
                : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
@@ -111,12 +105,6 @@ __device__ __forceinline__ uint4 bf16x8_to_f16x8(uint4 v) {
 
 __device__ __forceinline__ float2 ldcg2(const float* p) { return __ldcg(reinterpret_cast<const float2*>(p)); }
 __device__ __forceinline__ float4 ldcg4s(const float* p) { return __ldcg(reinterpret_cast<const float4*>(p)); }
-
-__device__ __forceinline__ unsigned long long pack_best(float v, int row) {
-  unsigned int fb = __float_as_uint(v);
-  fb = (fb & 0x80000000u) ? ~fb : (fb | 0x80000000u);           // order-preserving
-  return (static_cast<unsigned long long>(fb) << 32) | (0xffffffffu - static_cast<unsigned int>(row));   // ties -> lower row
-}
 
 // The joint window runs on tcgen05.  A = the CTA's W_out rows as IEEE half in
 // 128B-swizzled K-major slabs of 64 columns (88 rows stored per slab; the M = 128 instruction reads on into the next slab /

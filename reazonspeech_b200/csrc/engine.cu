@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <nvtx3/nvToolsExt.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdlib>
@@ -58,6 +59,26 @@ inline int conv_len(int n) { return n > 0 ? (n - 1) / 2 + 1 : 0; }   // floor di
 // 16-byte aligned: an odd T_max raised "illegal instruction" on the V^T tile loads of the attention kernel).
 inline int enc_capacity(int mel_frames) { return (conv_len(conv_len(conv_len(mel_frames))) + 7) & ~7; }
 
+// CUDA-event pairs around launches on their own streams, created on first use and reused after clear(); one
+// (tag, flops) entry per completed pair.
+struct EventLog {
+  bool on = false;
+  std::vector<cudaEvent_t> ev;
+  std::vector<std::pair<std::string, double>> entries;
+  void begin(cudaStream_t s) {
+    const size_t i = 2 * entries.size();
+    while (ev.size() < i + 2) { cudaEvent_t x; cudaEventCreate(&x); ev.push_back(x); }
+    cudaEventRecord(ev[i], s);
+  }
+  void end(cudaStream_t s, const std::string& tag, double flops) {
+    cudaEventRecord(ev[2 * entries.size() + 1], s);
+    entries.emplace_back(tag, flops);
+  }
+  float ms(size_t i) const { float t = 0.f; cudaEventElapsedTime(&t, ev[2 * i], ev[2 * i + 1]); return t; }
+  void clear() { entries.clear(); }
+  ~EventLog() { for (cudaEvent_t x : ev) cudaEventDestroy(x); }
+};
+
 }  // namespace
 
 struct rs_engine {
@@ -79,22 +100,14 @@ struct rs_engine {
   struct { const void *enc_w, *out_w, *lstm_w, *pred_w; const float *enc_b, *out_b, *embed, *lstm_b, *pred_b, *gate_tab; } dec;
   void* ws = nullptr;
   size_t ws_bytes = 0;
-  int U_cap = 0;
   mutable char err[512] = "";
   int64_t launches = 0;
   bool timing = false;
-  cudaEvent_t ev[9] = {};
+  cudaEvent_t ev[6] = {};               // stage marks of the whole path (rs_stage_times_ms)
   bool ev_ok = false;
-  float stage_ms[8] = {};
-  bool gemm_timing = false;
-  std::vector<cudaEvent_t> gemm_ev;     // pairs
-  size_t gemm_ev_used = 0;
-  double gemm_flops = 0.0;
+  EventLog gemm_log;                    // every GEMM launch, with its 2*M*N*K
   // per-kernel timing inside the real pipeline (warm caches, back-to-back launches): event pair around every launch
-  bool ktiming = false;
-  cudaStream_t cur_stream = nullptr;
-  std::vector<cudaEvent_t> k_ev;
-  std::vector<std::string> k_tag;       // one per event pair
+  EventLog kernel_log;
   // rs_transcribe_batch: host->device copies run on their own stream in utterance chunks so the frontend of
   // chunk i overlaps the copy of chunk i+1
   static constexpr int kCopyChunks = 8;
@@ -119,7 +132,11 @@ int fail(const rs_engine* e, int code, const char* fmt, ...) {
     if (_c != cudaSuccess) return fail((e), RS_ERR_CUDA, "%s: %s", #call, cudaGetErrorString(_c)); \
   } while (0)
 
-size_t align_up(size_t v) { return (v + 255) & ~static_cast<size_t>(255); }
+// Bump allocator of workspace offsets: every region starts 256-byte aligned; `off` ends as the total size.
+struct Arena {
+  size_t off = 0;
+  size_t take(size_t bytes) { const size_t o = off; off = (off + bytes + 255) & ~static_cast<size_t>(255); return o; }
+};
 
 inline size_t dec_ws_bytes(const rs_engine* e, int B) {
   return rs::rnnt_spec_workspace_bytes(B, e->cfg.joint_hidden, e->cfg.pred_hidden, e->num_sms);
@@ -136,34 +153,33 @@ Plan make_plan(const rs_engine* e, int B, int L_max, int U_max) {
   p.M = B * p.T3;
   const size_t C = c.sub_channels, d = c.d_model;
   const size_t wide = static_cast<size_t>(c.d_ff) > 3 * d ? c.d_ff : 3 * d;
-  size_t off = 0;
-  auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes); return o; };
-  p.wav = take(static_cast<size_t>(B) * L_max * 4);
-  p.len = take(static_cast<size_t>(B) * 4);
-  p.mel = take(static_cast<size_t>(B) * p.F_max * c.n_mels * 4);
-  p.mel_len = take(static_cast<size_t>(B) * 4);
-  p.mel_part = take(static_cast<size_t>(B) * rs::logmel_tiles(L_max, c.n_window_stride) * c.n_mels * 2 * 4);   // per-CTA (sum, sum of squares)
-  p.mel_stats = take(static_cast<size_t>(B) * c.n_mels * 2 * 4);                                               // (mean, 1 / (std + eps))
-  p.enc_len = take(static_cast<size_t>(B) * 4);
-  p.sub1 = take(static_cast<size_t>(B) * p.T2 * p.F2 * C * 2);
-  p.sub2 = take(static_cast<size_t>(B) * p.T2 * p.F2 * C * 2);
-  p.sub3 = take(static_cast<size_t>(B) * p.T3 * p.F3 * C * 2);
-  p.sub4 = take(static_cast<size_t>(B) * p.T3 * p.F3 * C * 2);
-  p.x = take(static_cast<size_t>(p.M) * d * 4);
-  p.xn = take(static_cast<size_t>(p.M) * d * 2);
-  p.hbuf = take(static_cast<size_t>(p.M) * wide * 2);
-  p.abuf = take(static_cast<size_t>(p.M) * d * 2);
-  p.cbuf = take(static_cast<size_t>(p.M) * d * 2);
+  Arena a;
+  p.wav = a.take(static_cast<size_t>(B) * L_max * 4);
+  p.len = a.take(static_cast<size_t>(B) * 4);
+  p.mel = a.take(static_cast<size_t>(B) * p.F_max * c.n_mels * 4);
+  p.mel_len = a.take(static_cast<size_t>(B) * 4);
+  p.mel_part = a.take(static_cast<size_t>(B) * rs::logmel_tiles(L_max, c.n_window_stride) * c.n_mels * 2 * 4);   // per-CTA (sum, sum of squares)
+  p.mel_stats = a.take(static_cast<size_t>(B) * c.n_mels * 2 * 4);                                               // (mean, 1 / (std + eps))
+  p.enc_len = a.take(static_cast<size_t>(B) * 4);
+  p.sub1 = a.take(static_cast<size_t>(B) * p.T2 * p.F2 * C * 2);
+  p.sub2 = a.take(static_cast<size_t>(B) * p.T2 * p.F2 * C * 2);
+  p.sub3 = a.take(static_cast<size_t>(B) * p.T3 * p.F3 * C * 2);
+  p.sub4 = a.take(static_cast<size_t>(B) * p.T3 * p.F3 * C * 2);
+  p.x = a.take(static_cast<size_t>(p.M) * d * 4);
+  p.xn = a.take(static_cast<size_t>(p.M) * d * 2);
+  p.hbuf = a.take(static_cast<size_t>(p.M) * wide * 2);
+  p.abuf = a.take(static_cast<size_t>(p.M) * d * 2);
+  p.cbuf = a.take(static_cast<size_t>(p.M) * d * 2);
   p.n_rel_pad = ((c.att_left + c.att_right + 1 + 31) / 32) * 32;
   p.ld_vt = ((p.M + 255) / 256) * 256 + 64;                               // V^T row pitch: covers the GEMM's 256-row tile overhang
-  p.vt = take(static_cast<size_t>(d) * p.ld_vt * 2);
-  p.enc = take(static_cast<size_t>(p.M) * d * 4);
-  p.encp = take(static_cast<size_t>(p.M) * c.joint_hidden * 4);
-  p.tokens = take(static_cast<size_t>(B) * U_max * 4);
-  p.frames = take(static_cast<size_t>(B) * U_max * 4);
-  p.ntok = take(static_cast<size_t>(B) * 4);
-  p.dec_ws = take(dec_ws_bytes(e, B));
-  p.total = off;
+  p.vt = a.take(static_cast<size_t>(d) * p.ld_vt * 2);
+  p.enc = a.take(static_cast<size_t>(p.M) * d * 4);
+  p.encp = a.take(static_cast<size_t>(p.M) * c.joint_hidden * 4);
+  p.tokens = a.take(static_cast<size_t>(B) * U_max * 4);
+  p.frames = a.take(static_cast<size_t>(B) * U_max * 4);
+  p.ntok = a.take(static_cast<size_t>(B) * 4);
+  p.dec_ws = a.take(dec_ws_bytes(e, B));
+  p.total = a.off;
   return p;
 }
 
@@ -256,70 +272,44 @@ __global__ void enc_len_kernel(const int32_t* __restrict__ mel_len, int32_t* __r
   enc_len[b] = n;
 }
 
-int gemm_args(rs_engine* e, const rs::GemmArgs& g, cudaStream_t s);
+#define RS_TRY(x) do { int _r = (x); if (_r != RS_OK) return _r; } while (0)
 
-int gemm(rs_engine* e, const void* a, const void* w, const float* bias, const float* resid, void* out, int M, int N,
-         int K, int epi, float alpha, cudaStream_t s) {
-  rs::GemmArgs g{a, w, bias, resid, out, M, N, K, epi, alpha};
-  return gemm_args(e, g, s);
-}
-
-void ktime_begin(rs_engine* e, const char* tag) {
-  if (!e->ktiming) return;
-  const size_t i = 2 * e->k_tag.size();
-  while (e->k_ev.size() < i + 2) { cudaEvent_t ev; cudaEventCreate(&ev); e->k_ev.push_back(ev); }
-  std::string t(tag);
-  if (t.rfind("rs::", 0) == 0) t = t.substr(4);
-  const size_t par = t.find('(');
-  e->k_tag.push_back(par == std::string::npos ? t : t.substr(0, par));
-  cudaEventRecord(e->k_ev[i], e->cur_stream);
-}
-void ktime_end(rs_engine* e) {
-  if (!e->ktiming) return;
-  cudaEventRecord(e->k_ev[2 * e->k_tag.size() - 1], e->cur_stream);
-}
-
-int gemm_args(rs_engine* e, const rs::GemmArgs& g_in, cudaStream_t s) {
-  const rs::GemmArgs& g = g_in;
-  const int M = g.M, N = g.N, K = g.K;
+// Every launch of the engine goes through here.  `call(msg)` enqueues `n` kernels on `s` and returns the CUDA error (msg, 256
+// bytes, may describe it better than the error's name).  Counts the launches, brackets the enqueue in the event logs that are
+// on (the GEMM log takes the launches with flops > 0) and turns a failure into fail("<tag>: <description>").  In the kernel
+// log the launch is named by `tag` without a leading "rs::" and without its argument list.
+template <typename Call>
+int launch(rs_engine* e, cudaStream_t s, const char* tag, int n, double flops, Call&& call) {
+  const bool klog = e->kernel_log.on, glog = flops > 0 && e->gemm_log.on;
+  if (glog) e->gemm_log.begin(s);
+  if (klog) e->kernel_log.begin(s);
   char msg[256] = "";
-  bool timed = false;
-  if (e->gemm_timing) {
-    if (e->gemm_ev_used + 2 > e->gemm_ev.size()) {
-      const size_t old = e->gemm_ev.size();
-      e->gemm_ev.resize(old + 512);
-      for (size_t i = old; i < e->gemm_ev.size(); ++i) cudaEventCreate(&e->gemm_ev[i]);
-    }
-    cudaEventRecord(e->gemm_ev[e->gemm_ev_used], s);
-    timed = true;
+  const cudaError_t c = call(msg);
+  if (c != cudaSuccess) return fail(e, RS_ERR_CUDA, "%s: %s", tag, msg[0] ? msg : cudaGetErrorString(c));
+  if (klog || glog) {
+    std::string name(tag);
+    if (name.rfind("rs::", 0) == 0) name = name.substr(4);
+    name = name.substr(0, name.find('('));
+    if (klog) e->kernel_log.end(s, name, 0.0);
+    if (glog) e->gemm_log.end(s, name, flops);
   }
-  if (e->ktiming) {
-    char tag[64];
-    snprintf(tag, sizeof tag, "gemm N=%d K=%d epi=%d%s", N, K, g.epilogue, g.n_batch > 1 ? " batched" : "");
-    e->cur_stream = s;
-    ktime_begin(e, tag);
-  }
-  cudaError_t c = rs::launch_gemm(g, e->num_sms, s, msg);
-  ktime_end(e);
-  if (c != cudaSuccess) return fail(e, RS_ERR_CUDA, "gemm: %s", msg);
-  if (timed) {
-    cudaEventRecord(e->gemm_ev[e->gemm_ev_used + 1], s);
-    e->gemm_ev_used += 2;
-    e->gemm_flops += 2.0 * M * static_cast<double>(N) * K * (g.n_batch > 0 ? g.n_batch : 1);
-  }
-  e->launches++;
+  e->launches += n;
   return RS_OK;
 }
 
-#define RS_TRY(x) do { int _r = (x); if (_r != RS_OK) return _r; } while (0)
-#define RS_K(e, call, n)                                                                       \
-  do {                                                                                         \
-    ktime_begin((e), #call);                                                                   \
-    cudaError_t _c = (call);                                                                   \
-    ktime_end((e));                                                                            \
-    if (_c != cudaSuccess) return fail((e), RS_ERR_CUDA, "%s: %s", #call, cudaGetErrorString(_c)); \
-    (e)->launches += (n);                                                                      \
-  } while (0)
+#define RS_K(e, s, call, n) RS_TRY(launch((e), (s), #call, (n), 0.0, [&](char*) { return (call); }))
+
+int gemm(rs_engine* e, const rs::GemmArgs& g, cudaStream_t s) {
+  char tag[64] = "gemm";
+  if (e->kernel_log.on) snprintf(tag, sizeof tag, "gemm N=%d K=%d epi=%d", g.N, g.K, g.epilogue);
+  return launch(e, s, tag, 1, 2.0 * g.M * static_cast<double>(g.N) * g.K,
+                [&](char* msg) { return rs::launch_gemm(g, e->num_sms, s, msg); });
+}
+
+int gemm(rs_engine* e, const void* a, const void* w, const float* bias, const float* resid, void* out, int M, int N,
+         int K, int epi, float alpha, cudaStream_t s) {
+  return gemm(e, rs::GemmArgs{a, w, bias, resid, out, M, N, K, epi, alpha}, s);
+}
 
 int check_ws(rs_engine* e, const Plan& p) {
   if (e->ws == nullptr) return fail(e, RS_ERR_WORKSPACE, "no workspace set (rs_set_workspace)");
@@ -337,7 +327,6 @@ void mark(rs_engine* e, int i, cudaStream_t s) {
 int do_logmel(rs_engine* e, const void* wav, bool i16, const int32_t* len, int nb, int L_max, float* mel, int32_t* mel_len,
               float* partials, float* stats, int b0, bool normalise, cudaStream_t s) {
   Nvtx range("rs::logmel");
-  e->cur_stream = s;
   const rs_model_config& c = e->cfg;
   if (b0 + nb > rs_engine::kMaxBatch) return fail(e, RS_ERR_INVALID_ARG, "batch of %d utterances exceeds the engine limit of %d", b0 + nb, rs_engine::kMaxBatch);
   rs::LogmelArgs a{};
@@ -347,37 +336,34 @@ int do_logmel(rs_engine* e, const void* wav, bool i16, const int32_t* len, int n
   a.tickets = e->lm_tickets + b0;
   a.tb = e->fe; a.n_mels = c.n_mels; a.hop = c.n_window_stride; a.n_fft = c.n_fft; a.win = c.n_window_size;
   a.preemph = c.preemph; a.guard = c.log_zero_guard; a.eps = c.norm_eps; a.normalise_in_place = normalise;
-  RS_K(e, rs::launch_logmel_fused(a, s), normalise ? 2 : 1);
+  RS_K(e, s, rs::launch_logmel_fused(a, s), normalise ? 2 : 1);
   return RS_OK;
 }
 
 // mel_stats == nullptr: `mel` is already normalised (rs_encode takes rs_logmel's output)
 int do_sub_conv0(rs_engine* e, const Plan& p, const float* mel, const int32_t* mel_len, const float* mel_stats, int b0, int nb, cudaStream_t s) {
   Nvtx range("rs::subsampling.conv0_dw1");
-  e->cur_stream = s;
   const rs_model_config& c = e->cfg;
   const int C = c.sub_channels;
   rs::SubsampleArgs sa{mel + static_cast<size_t>(b0) * p.F_max * c.n_mels, mel_len + b0,
                        mel_stats ? mel_stats + static_cast<size_t>(b0) * c.n_mels * 2 : nullptr, nb, p.F_max, c.n_mels, C,
                        e->sub.c0w, e->sub.c0b, e->sub.d1w, e->sub.d1b,
                        at<uint16_t>(e, p.sub1) + static_cast<size_t>(b0) * p.T2 * p.F2 * C, p.T1, p.F1, p.T2, p.F2};
-  RS_K(e, rs::launch_sub_conv0_dw1(sa, s), 1);
+  RS_K(e, s, rs::launch_sub_conv0_dw1(sa, s), 1);
   return RS_OK;
 }
 
-int do_encode(rs_engine* e, const Plan& p, const float* mel, const int32_t* mel_len, const float* mel_stats, float* enc, int32_t* enc_len,
-              int n_layers, cudaStream_t s, bool conv0_done = false) {
-  e->cur_stream = s;
+// The encoder after the first (fused) subsampling conv, which the caller has run into p.sub1.
+int do_encode(rs_engine* e, const Plan& p, const int32_t* mel_len, float* enc, int32_t* enc_len, int n_layers, cudaStream_t s) {
   const rs_model_config& c = e->cfg;
   const int d = c.d_model, C = c.sub_channels, M = p.M, B = p.B;
   if (n_layers < 0 || n_layers > c.n_layers) n_layers = c.n_layers;
   enc_len_kernel<<<(B + 127) / 128, 128, 0, s>>>(mel_len, enc_len, B);
-  RS_K(e, cudaGetLastError(), 1);
+  RS_K(e, s, cudaGetLastError(), 1);
   // ---- ConvSubsampling
-  if (!conv0_done) RS_TRY(do_sub_conv0(e, p, mel, mel_len, mel_stats, 0, B, s));
   RS_TRY(gemm(e, at<void>(e, p.sub1), e->sub.p1w, e->sub.p1b, nullptr, at<void>(e, p.sub2), B * p.T2 * p.F2, C, C,
               RS_EPI_BIAS_RELU_BF16, 1.f, s));
-  RS_K(e, rs::launch_sub_dw(at<void>(e, p.sub2), at<void>(e, p.sub3), e->sub.d2w, e->sub.d2b, mel_len, 2, B, p.T2, p.F2,
+  RS_K(e, s, rs::launch_sub_dw(at<void>(e, p.sub2), at<void>(e, p.sub3), e->sub.d2w, e->sub.d2b, mel_len, 2, B, p.T2, p.F2,
                             p.T3, p.F3, C, s), 1);
   RS_TRY(gemm(e, at<void>(e, p.sub3), e->sub.p2w, e->sub.p2b, nullptr, at<void>(e, p.sub4), B * p.T3 * p.F3, C, C,
               RS_EPI_BIAS_RELU_BF16, 1.f, s));
@@ -389,7 +375,7 @@ int do_encode(rs_engine* e, const Plan& p, const float* mel, const int32_t* mel_
   void* xn = at<void>(e, p.xn); void* hb = at<void>(e, p.hbuf); void* ab = at<void>(e, p.abuf); void* cb = at<void>(e, p.cbuf);
   if (n_layers > 0) {
     const LayerW& L0 = e->layers[0];
-    RS_K(e, rs::launch_layernorm(x, L0.ln_ff1_g, L0.ln_ff1_b, nullptr, xn, nullptr, nullptr, M, d, c.ln_eps, s), 1);
+    RS_K(e, s, rs::launch_layernorm(x, L0.ln_ff1_g, L0.ln_ff1_b, nullptr, xn, nullptr, nullptr, M, d, c.ln_eps, s), 1);
   }
   auto resid_gemm = [&](const void* a, const void* w, const float* bias, int K, float alpha) -> int {
     return gemm(e, a, w, bias, x, x, M, d, K, RS_EPI_RESID_F32, alpha, s);
@@ -401,43 +387,42 @@ int do_encode(rs_engine* e, const Plan& p, const float* mel, const int32_t* mel_
     Nvtx layer_range(layer_name);
     RS_TRY(gemm(e, xn, L.ff1_w1, L.ff1_b1, nullptr, hb, M, c.d_ff, d, RS_EPI_BIAS_SWISH_BF16, 1.f, s));
     RS_TRY(resid_gemm(hb, L.ff1_w2, L.ff1_b2, c.d_ff, 0.5f));
-    RS_K(e, rs::launch_layernorm(x, L.ln_att_g, L.ln_att_b, nullptr, xn, nullptr, nullptr, M, d, c.ln_eps, s), 1);
+    RS_K(e, s, rs::launch_layernorm(x, L.ln_att_g, L.ln_att_b, nullptr, xn, nullptr, nullptr, M, d, c.ln_eps, s), 1);
     // the relative-position term (q + pos_bias_v) . p[c] is a UMMA inside the attention kernel (attention_tc.cu): no score tensor in HBM
     rs::AttnArgs aa{hb, L.att_pos, L.att_bdbias, p.n_rel_pad, L.att_u, ab, enc_len, B, p.T3, c.n_heads, d / c.n_heads, c.att_left, c.att_right, c.global_tokens};
     aa.vt = at<void>(e, p.vt); aa.ld_vt = p.ld_vt;
     {   // q | k row-major, V transposed (keys contiguous) for the attention's P.V product
       rs::GemmArgs g{xn, L.wqkv, L.bqkv, nullptr, hb, M, 3 * d, d, RS_EPI_QKV_VT, 1.f};
       g.out2 = at<void>(e, p.vt); g.split = 2 * d; g.ld2 = p.ld_vt;
-      RS_TRY(gemm_args(e, g, s));
+      RS_TRY(gemm(e, g, s));
     }
-    RS_K(e, rs::launch_attention_tc(aa, s), c.global_tokens > 0 ? 2 : 1);
+    RS_K(e, s, rs::launch_attention_tc(aa, s), c.global_tokens > 0 ? 2 : 1);
     RS_TRY(resid_gemm(ab, L.wo, L.bo, d, 1.f));
-    RS_K(e, rs::launch_layernorm(x, L.ln_conv_g, L.ln_conv_b, nullptr, xn, nullptr, nullptr, M, d, c.ln_eps, s), 1);
+    RS_K(e, s, rs::launch_layernorm(x, L.ln_conv_g, L.ln_conv_b, nullptr, xn, nullptr, nullptr, M, d, c.ln_eps, s), 1);
     RS_TRY(gemm(e, xn, L.pw1_w, L.pw1_b, nullptr, ab, M, 2 * d, d, RS_EPI_BIAS_GLU_BF16, 1.f, s));
-    RS_K(e, rs::launch_conv_dw(ab, cb, L.dw_w, L.dw_shift, enc_len, B, p.T3, d, c.conv_kernel, s), 1);
+    RS_K(e, s, rs::launch_conv_dw(ab, cb, L.dw_w, L.dw_shift, enc_len, B, p.T3, d, c.conv_kernel, s), 1);
     RS_TRY(resid_gemm(cb, L.pw2_w, L.pw2_b, d, 1.f));
-    RS_K(e, rs::launch_layernorm(x, L.ln_ff2_g, L.ln_ff2_b, nullptr, xn, nullptr, nullptr, M, d, c.ln_eps, s), 1);
+    RS_K(e, s, rs::launch_layernorm(x, L.ln_ff2_g, L.ln_ff2_b, nullptr, xn, nullptr, nullptr, M, d, c.ln_eps, s), 1);
     RS_TRY(gemm(e, xn, L.ff2_w1, L.ff2_b1, nullptr, hb, M, c.d_ff, d, RS_EPI_BIAS_SWISH_BF16, 1.f, s));
     RS_TRY(resid_gemm(hb, L.ff2_w2, L.ff2_b2, c.d_ff, 0.5f));
     if (i + 1 < n_layers) {   // norm_out chained with the next layer's norm_feed_forward1
       const LayerW& Ln = e->layers[i + 1];
-      RS_K(e, rs::launch_layernorm(x, L.ln_out_g, L.ln_out_b, x, xn, Ln.ln_ff1_g, Ln.ln_ff1_b, M, d, c.ln_eps, s), 1);
+      RS_K(e, s, rs::launch_layernorm(x, L.ln_out_g, L.ln_out_b, x, xn, Ln.ln_ff1_g, Ln.ln_ff1_b, M, d, c.ln_eps, s), 1);
     } else {
-      RS_K(e, rs::launch_layernorm(x, L.ln_out_g, L.ln_out_b, enc, nullptr, nullptr, nullptr, M, d, c.ln_eps, s), 1);
+      RS_K(e, s, rs::launch_layernorm(x, L.ln_out_g, L.ln_out_b, enc, nullptr, nullptr, nullptr, M, d, c.ln_eps, s), 1);
     }
   }
   if (n_layers == 0) RS_CUDA(e, cudaMemcpyAsync(enc, x, static_cast<size_t>(M) * d * 4, cudaMemcpyDeviceToDevice, s));
-  RS_K(e, rs::launch_zero_pad_rows(enc, enc_len, B, p.T3, d, s), 1);
+  RS_K(e, s, rs::launch_zero_pad_rows(enc, enc_len, B, p.T3, d, s), 1);
   return RS_OK;
 }
 
 int do_greedy(rs_engine* e, const Plan& p, const float* enc, const int32_t* enc_len, int T_max, int32_t* tokens,
               int32_t* frames, int32_t* ntok, int U_max, cudaStream_t s) {
   Nvtx range("rs::rnnt_greedy (joint.enc projection + persistent decode)");
-  e->cur_stream = s;
   const rs_model_config& c = e->cfg;
   const int M = p.B * T_max;
-  RS_K(e, rs::launch_f32_to_bf16(enc, at<void>(e, p.xn), static_cast<int64_t>(M) * c.d_model, s), 1);
+  RS_K(e, s, rs::launch_f32_to_bf16(enc, at<void>(e, p.xn), static_cast<int64_t>(M) * c.d_model, s), 1);
   RS_TRY(gemm(e, at<void>(e, p.xn), e->dec.enc_w, e->dec.enc_b, nullptr, at<void>(e, p.encp), M, c.joint_hidden, c.d_model,
               RS_EPI_BIAS_F32, 1.f, s));
   mark(e, 4, s);
@@ -447,8 +432,74 @@ int do_greedy(rs_engine* e, const Plan& p, const float* enc, const int32_t* enc_
   // One decode kernel for every batch size (windowed, weights-stationary, joint on tcgen05: decode_spec.cu): an utterance's
   // logits are accumulated in the same order whether it is decoded alone or inside a batch, so results do not depend on
   // batch composition.
-  RS_K(e, rs::launch_rnnt_greedy_spec(da, at<void>(e, p.dec_ws), e->num_sms, s), 2);
+  RS_K(e, s, rs::launch_rnnt_greedy_spec(da, at<void>(e, p.dec_ws), e->num_sms, s), 2);
   return RS_OK;
+}
+
+// The whole path.  chunks == 0: wav / len and the outputs are device pointers, nothing synchronises.  chunks >= 1: they are
+// host buffers; wav / len are copied into the workspace in `chunks` utterance chunks -- on the copy stream when there are
+// several, so that log-mel and the first (fused) subsampling conv of a chunk that has landed overlap the copy of the next --
+// and the results are copied back before the call synchronises.  `wav` holds f32 samples, or int16 PCM (scaled by 2^-15
+// inside the log-mel kernel) when i16.
+int transcribe(rs_engine* e, const void* wav_in, bool i16, const int32_t* len_in, int B, int L_max, int32_t* tokens,
+               int32_t* frames, int32_t* n_tok, int U_max, int chunks, cudaStream_t s) {
+  Plan p = make_plan(e, B, L_max, U_max);
+  RS_TRY(check_ws(e, p));
+  const bool host = chunks > 0;
+  const size_t esz = i16 ? 2 : 4;                       // the waveform region of the workspace is sized for f32
+  const char* wav = host ? at<char>(e, p.wav) : static_cast<const char*>(wav_in);
+  const int32_t* len = host ? at<int32_t>(e, p.len) : len_in;
+  const int per = host ? (B + chunks - 1) / chunks : B;
+  const cudaStream_t cs = chunks > 1 ? e->copy_stream : s;
+  if (host) {
+    if (cs != s) {   // the workspace may still be in use by work already queued on the caller's stream
+      RS_CUDA(e, cudaEventRecord(e->copy_ev[rs_engine::kCopyChunks], s));
+      RS_CUDA(e, cudaStreamWaitEvent(cs, e->copy_ev[rs_engine::kCopyChunks], 0));
+    }
+    RS_CUDA(e, cudaMemcpyAsync(at<int32_t>(e, p.len), len_in, static_cast<size_t>(B) * 4, cudaMemcpyHostToDevice, cs));
+    for (int c = 0, b0 = 0; b0 < B; ++c, b0 += per) {
+      const size_t off = static_cast<size_t>(b0) * L_max * esz, bytes = static_cast<size_t>(std::min(per, B - b0)) * L_max * esz;
+      RS_CUDA(e, cudaMemcpyAsync(at<char>(e, p.wav) + off, static_cast<const char*>(wav_in) + off, bytes, cudaMemcpyHostToDevice, cs));
+      if (cs != s) RS_CUDA(e, cudaEventRecord(e->copy_ev[c], cs));
+    }
+  }
+  float* mel = at<float>(e, p.mel);
+  int32_t* mel_len = at<int32_t>(e, p.mel_len);
+  float* stats = at<float>(e, p.mel_stats);
+  mark(e, 0, s);
+  for (int c = 0, b0 = 0; b0 < B; ++c, b0 += per) {
+    const int nb = std::min(per, B - b0);
+    if (cs != s) RS_CUDA(e, cudaStreamWaitEvent(s, e->copy_ev[c], 0));
+    RS_TRY(do_logmel(e, wav + static_cast<size_t>(b0) * L_max * esz, i16, len + b0, nb, L_max,
+                     mel + static_cast<size_t>(b0) * p.F_max * e->cfg.n_mels, mel_len + b0, at<float>(e, p.mel_part), stats, b0, false, s));
+    if (b0 + nb == B) mark(e, 1, s);
+    RS_TRY(do_sub_conv0(e, p, mel, mel_len, stats, b0, nb, s));
+  }
+  RS_TRY(do_encode(e, p, mel_len, at<float>(e, p.enc), at<int32_t>(e, p.enc_len), -1, s));
+  mark(e, 3, s);
+  int32_t* tok = host ? at<int32_t>(e, p.tokens) : tokens;
+  int32_t* frm = host ? at<int32_t>(e, p.frames) : frames;
+  int32_t* cnt = host ? at<int32_t>(e, p.ntok) : n_tok;
+  RS_TRY(do_greedy(e, p, at<float>(e, p.enc), at<int32_t>(e, p.enc_len), p.T3, tok, frm, cnt, U_max, s));
+  mark(e, 5, s);
+  if (host) {
+    RS_CUDA(e, cudaMemcpyAsync(tokens, tok, static_cast<size_t>(B) * U_max * 4, cudaMemcpyDeviceToHost, s));
+    RS_CUDA(e, cudaMemcpyAsync(frames, frm, static_cast<size_t>(B) * U_max * 4, cudaMemcpyDeviceToHost, s));
+    RS_CUDA(e, cudaMemcpyAsync(n_tok, cnt, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, s));
+    RS_CUDA(e, cudaStreamSynchronize(s));
+  }
+  return RS_OK;
+}
+
+// The four rs_transcribe_* entry points: argument check, device, and the host entries' chunk rule (kCopyChunks chunks on
+// the copy stream from 2 * kCopyChunks utterances on, else one on the caller's stream).
+int transcribe_entry(const char* name, rs_engine* e, const void* wav, bool i16, const int32_t* len, int B, int L_max,
+                     int32_t* tokens, int32_t* frames, int32_t* n_tok, int U_max, bool host, void* stream) {
+  if (!e || !wav || !len || !tokens || !frames || !n_tok || B <= 0 || L_max <= 0 || U_max <= 0)
+    return fail(e, RS_ERR_INVALID_ARG, "%s: bad arguments", name);
+  RS_CUDA(e, cudaSetDevice(e->device));
+  const int chunks = !host ? 0 : (e->copy_ok && B >= 2 * rs_engine::kCopyChunks) ? rs_engine::kCopyChunks : 1;
+  return transcribe(e, wav, i16, len, B, L_max, tokens, frames, n_tok, U_max, chunks, static_cast<cudaStream_t>(stream));
 }
 
 }  // namespace
@@ -503,8 +554,6 @@ void rs_engine_destroy(rs_engine* e) {
   if (e->ev_ok) for (auto& ev : e->ev) cudaEventDestroy(ev);
   for (auto& ev : e->copy_ev) if (ev) cudaEventDestroy(ev);
   if (e->copy_stream) cudaStreamDestroy(e->copy_stream);
-  for (auto& ev : e->gemm_ev) cudaEventDestroy(ev);
-  for (auto& ev : e->k_ev) cudaEventDestroy(ev);
   cudaFree(e->lm_tickets);
   cudaFree(e->alsd_ws);
   if (e->alsd_done_host) cudaFreeHost(e->alsd_done_host);
@@ -549,7 +598,9 @@ int rs_encode(rs_engine* e, const float* mel, const int32_t* mel_len, int B, int
   const int L_max = (F_max - 1) * e->cfg.n_window_stride;
   Plan p = make_plan(e, B, L_max, 1);
   RS_TRY(check_ws(e, p));
-  return do_encode(e, p, mel, mel_len, nullptr, enc, enc_len, n_layers, static_cast<cudaStream_t>(stream));
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  RS_TRY(do_sub_conv0(e, p, mel, mel_len, nullptr, 0, B, s));
+  return do_encode(e, p, mel_len, enc, enc_len, n_layers, s);
 }
 
 int rs_rnnt_greedy(rs_engine* e, const float* enc, const int32_t* enc_len, int B, int T_max, int32_t* tokens,
@@ -558,120 +609,37 @@ int rs_rnnt_greedy(rs_engine* e, const float* enc, const int32_t* enc_len, int B
     return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_greedy: bad arguments");
   RS_CUDA(e, cudaSetDevice(e->device));
   Plan p{};
-  // only xn / encp are touched: size them for M = B*T_max rows
+  // only xn / encp / dec_ws are touched: size them for M = B*T_max rows
   p.B = B; p.M = B * T_max;
-  size_t off = 0;
-  p.xn = off; off = align_up(off + static_cast<size_t>(p.M) * e->cfg.d_model * 2);
-  p.encp = off; off = align_up(off + static_cast<size_t>(p.M) * e->cfg.joint_hidden * 4);
-  p.dec_ws = off; off = align_up(off + dec_ws_bytes(e, B));
-  p.total = off; p.L_max = 0;
+  Arena a;
+  p.xn = a.take(static_cast<size_t>(p.M) * e->cfg.d_model * 2);
+  p.encp = a.take(static_cast<size_t>(p.M) * e->cfg.joint_hidden * 4);
+  p.dec_ws = a.take(dec_ws_bytes(e, B));
+  p.total = a.off;
   RS_TRY(check_ws(e, p));
   return do_greedy(e, p, enc, enc_len, T_max, tokens, frames, n_tok, U_max, static_cast<cudaStream_t>(stream));
 }
 
-}  // extern "C"
-
-namespace {
-
-// Device-resident whole path; `wav` holds f32 samples, or int16 PCM (scaled by 2^-15 inside the log-mel kernel) when i16.
-int transcribe_device(rs_engine* e, const void* wav, bool i16, const int32_t* len, int B, int L_max, int32_t* tokens,
-                      int32_t* frames, int32_t* n_tok, int U_max, cudaStream_t s) {
-  Plan p = make_plan(e, B, L_max, U_max);
-  RS_TRY(check_ws(e, p));
-  mark(e, 0, s);
-  RS_TRY(do_logmel(e, wav, i16, len, B, L_max, at<float>(e, p.mel), at<int32_t>(e, p.mel_len), at<float>(e, p.mel_part), at<float>(e, p.mel_stats), 0, false, s));
-  mark(e, 1, s);
-  RS_TRY(do_encode(e, p, at<float>(e, p.mel), at<int32_t>(e, p.mel_len), at<float>(e, p.mel_stats), at<float>(e, p.enc), at<int32_t>(e, p.enc_len), -1, s));
-  mark(e, 3, s);
-  RS_TRY(do_greedy(e, p, at<float>(e, p.enc), at<int32_t>(e, p.enc_len), p.T3, tokens, frames, n_tok, U_max, s));
-  mark(e, 5, s);
-  return RS_OK;
-}
-
-// Host buffers in, host buffers out (the model.transcribe seam): H2D in utterance chunks on the copy stream, overlapped with
-// the frontend of the chunks that have landed; D2H of the tokens; synchronises before returning.
-int transcribe_batch(rs_engine* e, const void* wav_host, bool i16, const int32_t* len_host, int B, int L_max,
-                     int32_t* tokens_host, int32_t* frames_host, int32_t* n_tok_host, int U_max, cudaStream_t s) {
-  Plan p = make_plan(e, B, L_max, U_max);
-  RS_TRY(check_ws(e, p));
-  const size_t esz = i16 ? 2 : 4;                       // the waveform region of the workspace is sized for f32
-  char* wav = at<char>(e, p.wav);
-  const char* wav_h = static_cast<const char*>(wav_host);
-  int32_t* len = at<int32_t>(e, p.len);
-  float* mel = at<float>(e, p.mel);
-  int32_t* mel_len = at<int32_t>(e, p.mel_len);
-  const int n_chunks = (e->copy_ok && B >= 2 * rs_engine::kCopyChunks) ? rs_engine::kCopyChunks : 1;
-  if (n_chunks == 1) {
-    RS_CUDA(e, cudaMemcpyAsync(wav, wav_h, static_cast<size_t>(B) * L_max * esz, cudaMemcpyHostToDevice, s));
-    RS_CUDA(e, cudaMemcpyAsync(len, len_host, static_cast<size_t>(B) * 4, cudaMemcpyHostToDevice, s));
-    RS_TRY(transcribe_device(e, wav, i16, len, B, L_max, at<int32_t>(e, p.tokens), at<int32_t>(e, p.frames),
-                             at<int32_t>(e, p.ntok), U_max, s));
-  } else {
-    // copies on the copy stream, chunk by chunk; log-mel and the first (fused) subsampling conv of a chunk start as
-    // soon as its samples have landed.  The copy stream first waits for everything already queued on the caller's
-    // stream (the workspace may still be in use by an earlier asynchronous call).
-    const int per = (B + n_chunks - 1) / n_chunks;
-    RS_CUDA(e, cudaEventRecord(e->copy_ev[n_chunks], s));
-    RS_CUDA(e, cudaStreamWaitEvent(e->copy_stream, e->copy_ev[n_chunks], 0));
-    RS_CUDA(e, cudaMemcpyAsync(len, len_host, static_cast<size_t>(B) * 4, cudaMemcpyHostToDevice, e->copy_stream));
-    for (int c = 0, b0 = 0; b0 < B; ++c, b0 += per) {
-      const int nb = (B - b0 < per) ? B - b0 : per;
-      RS_CUDA(e, cudaMemcpyAsync(wav + static_cast<size_t>(b0) * L_max * esz, wav_h + static_cast<size_t>(b0) * L_max * esz,
-                                 static_cast<size_t>(nb) * L_max * esz, cudaMemcpyHostToDevice, e->copy_stream));
-      RS_CUDA(e, cudaEventRecord(e->copy_ev[c], e->copy_stream));
-    }
-    for (int c = 0, b0 = 0; b0 < B; ++c, b0 += per) {
-      const int nb = (B - b0 < per) ? B - b0 : per;
-      RS_CUDA(e, cudaStreamWaitEvent(s, e->copy_ev[c], 0));
-      RS_TRY(do_logmel(e, wav + static_cast<size_t>(b0) * L_max * esz, i16, len + b0, nb, L_max,
-                       mel + static_cast<size_t>(b0) * p.F_max * e->cfg.n_mels, mel_len + b0, at<float>(e, p.mel_part), at<float>(e, p.mel_stats), b0, false, s));
-      RS_TRY(do_sub_conv0(e, p, mel, mel_len, at<float>(e, p.mel_stats), b0, nb, s));
-    }
-    RS_TRY(do_encode(e, p, mel, mel_len, at<float>(e, p.mel_stats), at<float>(e, p.enc), at<int32_t>(e, p.enc_len), -1, s, true));
-    RS_TRY(do_greedy(e, p, at<float>(e, p.enc), at<int32_t>(e, p.enc_len), p.T3, at<int32_t>(e, p.tokens),
-                     at<int32_t>(e, p.frames), at<int32_t>(e, p.ntok), U_max, s));
-  }
-  RS_CUDA(e, cudaMemcpyAsync(tokens_host, at<int32_t>(e, p.tokens), static_cast<size_t>(B) * U_max * 4, cudaMemcpyDeviceToHost, s));
-  RS_CUDA(e, cudaMemcpyAsync(frames_host, at<int32_t>(e, p.frames), static_cast<size_t>(B) * U_max * 4, cudaMemcpyDeviceToHost, s));
-  RS_CUDA(e, cudaMemcpyAsync(n_tok_host, at<int32_t>(e, p.ntok), static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, s));
-  RS_CUDA(e, cudaStreamSynchronize(s));
-  return RS_OK;
-}
-
-}  // namespace
-
-extern "C" {
-
 int rs_transcribe_device(rs_engine* e, const float* wav, const int32_t* len, int B, int L_max, int32_t* tokens,
                          int32_t* frames, int32_t* n_tok, int U_max, void* stream) {
-  if (!e || !wav || !len || !tokens || !frames || !n_tok || B <= 0 || L_max <= 0 || U_max <= 0)
-    return fail(e, RS_ERR_INVALID_ARG, "rs_transcribe_device: bad arguments");
-  RS_CUDA(e, cudaSetDevice(e->device));
-  return transcribe_device(e, wav, false, len, B, L_max, tokens, frames, n_tok, U_max, static_cast<cudaStream_t>(stream));
+  return transcribe_entry("rs_transcribe_device", e, wav, false, len, B, L_max, tokens, frames, n_tok, U_max, false, stream);
 }
 
 int rs_transcribe_device_pcm16(rs_engine* e, const int16_t* wav, const int32_t* len, int B, int L_max, int32_t* tokens,
                                int32_t* frames, int32_t* n_tok, int U_max, void* stream) {
-  if (!e || !wav || !len || !tokens || !frames || !n_tok || B <= 0 || L_max <= 0 || U_max <= 0)
-    return fail(e, RS_ERR_INVALID_ARG, "rs_transcribe_device_pcm16: bad arguments");
-  RS_CUDA(e, cudaSetDevice(e->device));
-  return transcribe_device(e, wav, true, len, B, L_max, tokens, frames, n_tok, U_max, static_cast<cudaStream_t>(stream));
+  return transcribe_entry("rs_transcribe_device_pcm16", e, wav, true, len, B, L_max, tokens, frames, n_tok, U_max, false, stream);
 }
 
 int rs_transcribe_batch(rs_engine* e, const float* wav_host, const int32_t* len_host, int B, int L_max,
                         int32_t* tokens_host, int32_t* frames_host, int32_t* n_tok_host, int U_max, void* stream) {
-  if (!e || !wav_host || !len_host || !tokens_host || !frames_host || !n_tok_host || B <= 0 || L_max <= 0 || U_max <= 0)
-    return fail(e, RS_ERR_INVALID_ARG, "rs_transcribe_batch: bad arguments");
-  RS_CUDA(e, cudaSetDevice(e->device));
-  return transcribe_batch(e, wav_host, false, len_host, B, L_max, tokens_host, frames_host, n_tok_host, U_max, static_cast<cudaStream_t>(stream));
+  return transcribe_entry("rs_transcribe_batch", e, wav_host, false, len_host, B, L_max, tokens_host, frames_host, n_tok_host,
+                          U_max, true, stream);
 }
 
 int rs_transcribe_batch_pcm16(rs_engine* e, const int16_t* wav_host, const int32_t* len_host, int B, int L_max,
                               int32_t* tokens_host, int32_t* frames_host, int32_t* n_tok_host, int U_max, void* stream) {
-  if (!e || !wav_host || !len_host || !tokens_host || !frames_host || !n_tok_host || B <= 0 || L_max <= 0 || U_max <= 0)
-    return fail(e, RS_ERR_INVALID_ARG, "rs_transcribe_batch_pcm16: bad arguments");
-  RS_CUDA(e, cudaSetDevice(e->device));
-  return transcribe_batch(e, wav_host, true, len_host, B, L_max, tokens_host, frames_host, n_tok_host, U_max, static_cast<cudaStream_t>(stream));
+  return transcribe_entry("rs_transcribe_batch_pcm16", e, wav_host, true, len_host, B, L_max, tokens_host, frames_host,
+                          n_tok_host, U_max, true, stream);
 }
 
 // ALSD beam search over encoder outputs (decode_alsd.cu; semantics: oracle/alsd_restated.py).  Synchronises: the host checks every
@@ -685,22 +653,20 @@ int rs_rnnt_alsd(rs_engine* e, const float* enc, const int32_t* enc_len, int B, 
   RS_CUDA(e, cudaSetDevice(e->device));
   Nvtx range("rs::rnnt_alsd");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  e->cur_stream = s;
   const rs_model_config& c = e->cfg;
   const int Hj = c.joint_hidden, Hp = c.pred_hidden, d = c.d_model, V = c.vocab_size, blank = c.vocab_size, n_pad = e->alsd.n_pad;
   const int M = B * T_max, R = B * beam;
   const int total_steps = T_max + static_cast<int>(u_max_ratio * static_cast<float>(T_max));
   const int max_nodes = 1 + beam * (total_steps + 1);
   // ---- workspace
-  size_t off = 0;
-  auto take = [&](size_t bytes) { off = align_up(off); size_t o = off; off += bytes; return o; };
-  const size_t o_xn = take(static_cast<size_t>(M) * d * 2), o_encp = take(static_cast<size_t>(M) * Hj * 4);
+  Arena a;
+  const size_t o_xn = a.take(static_cast<size_t>(M) * d * 2), o_encp = a.take(static_cast<size_t>(M) * Hj * 4);
   const size_t plane_cols = static_cast<size_t>(3 * Hj > 6 * Hp ? 3 * Hj : 6 * Hp);
-  const size_t o_planes = take(static_cast<size_t>(R) * plane_cols * 2), o_logits = take(static_cast<size_t>(R) * n_pad * 4);
-  const size_t o_gates = take(static_cast<size_t>(R) * 4 * Hp * 4), o_pp = take(static_cast<size_t>(R) * Hj * 4);
+  const size_t o_planes = a.take(static_cast<size_t>(R) * plane_cols * 2), o_logits = a.take(static_cast<size_t>(R) * n_pad * 4);
+  const size_t o_gates = a.take(static_cast<size_t>(R) * 4 * Hp * 4), o_pp = a.take(static_cast<size_t>(R) * Hj * 4);
   const size_t state_bytes = rs::alsd_state_bytes(B, beam, Hp, Hj, max_nodes);
-  const size_t o_state = take(state_bytes);
-  const size_t need_bytes = align_up(off);
+  const size_t o_state = a.take(state_bytes);
+  const size_t need_bytes = a.off;
   if (need_bytes > e->alsd_ws_bytes) {
     RS_CUDA(e, cudaStreamSynchronize(s));
     cudaFree(e->alsd_ws); e->alsd_ws = nullptr; e->alsd_ws_bytes = 0;
@@ -715,24 +681,24 @@ int rs_rnnt_alsd(rs_engine* e, const float* enc, const int32_t* enc_len, int B, 
   rs::AlsdState st{};
   rs::alsd_bind_state(st, ws + o_state, B, beam, Hp, Hj, max_nodes, score_norm != 0);
   // ---- joint.enc over every frame (as in the greedy path)
-  RS_K(e, rs::launch_f32_to_bf16(enc, xn, static_cast<int64_t>(M) * d, s), 1);
+  RS_K(e, s, rs::launch_f32_to_bf16(enc, xn, static_cast<int64_t>(M) * d, s), 1);
   RS_TRY(gemm(e, xn, e->dec.enc_w, e->dec.enc_b, nullptr, encp, M, Hj, d, RS_EPI_BIAS_F32, 1.f, s));
   // predictor of the extended hypotheses of the beam being built (also the start: [blank] from the zero state)
   auto predictor = [&]() -> int {
-    RS_K(e, rs::alsd_launch_lstm_in(st, B, e->dec.embed, Hp, planes, s), 1);
+    RS_K(e, s, rs::alsd_launch_lstm_in(st, B, e->dec.embed, Hp, planes, s), 1);
     RS_TRY(gemm(e, planes, e->alsd.lstm_w3, e->dec.lstm_b, nullptr, gates, R, 4 * Hp, 6 * Hp, RS_EPI_BIAS_F32, 1.f, s));
-    RS_K(e, rs::alsd_launch_cell(st, B, gates, Hp, planes, s), 1);
+    RS_K(e, s, rs::alsd_launch_cell(st, B, gates, Hp, planes, s), 1);
     RS_TRY(gemm(e, planes, e->alsd.pred_w3, e->dec.pred_b, nullptr, ppn, R, Hj, 3 * Hp, RS_EPI_BIAS_F32, 1.f, s));
-    RS_K(e, rs::alsd_launch_commit(st, B, ppn, Hp, Hj, s), 2);
+    RS_K(e, s, rs::alsd_launch_commit(st, B, ppn, Hp, Hj, s), 2);
     return RS_OK;
   };
-  RS_K(e, rs::alsd_launch_init(st, B, blank, s), 1);
+  RS_K(e, s, rs::alsd_launch_init(st, B, blank, s), 1);
   RS_TRY(predictor());
   for (int step = 0; step <= total_steps; ++step) {
-    RS_K(e, rs::alsd_launch_rows(st, B, encp, enc_len, T_max, Hj, step, planes, s), 1);
+    RS_K(e, s, rs::alsd_launch_rows(st, B, encp, enc_len, T_max, Hj, step, planes, s), 1);
     RS_TRY(gemm(e, planes, e->alsd.out_w3, e->alsd.out_b, nullptr, logits, R, n_pad, 3 * Hj, RS_EPI_BIAS_F32, 1.f, s));
-    RS_K(e, rs::alsd_launch_reduce(st, B, logits, n_pad, V, s), 1);
-    RS_K(e, rs::alsd_launch_select(st, B, enc_len, step, blank, u_max_ratio, recombine_returns_input != 0, s), 1);
+    RS_K(e, s, rs::alsd_launch_reduce(st, B, logits, n_pad, V, s), 1);
+    RS_K(e, s, rs::alsd_launch_select(st, B, enc_len, step, blank, u_max_ratio, recombine_returns_input != 0, s), 1);
     RS_TRY(predictor());
     if ((step & 31) == 31) {
       RS_CUDA(e, cudaMemcpyAsync(e->alsd_done_host, st.n_done, sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -740,7 +706,7 @@ int rs_rnnt_alsd(rs_engine* e, const float* enc, const int32_t* enc_len, int B, 
       if (*e->alsd_done_host >= B) break;
     }
   }
-  RS_K(e, rs::alsd_launch_output(st, B, blank, y_dev, step_dev, n_dev, score_dev, U_cap, s), 1);
+  RS_K(e, s, rs::alsd_launch_output(st, B, blank, y_dev, step_dev, n_dev, score_dev, U_cap, s), 1);
   RS_CUDA(e, cudaStreamSynchronize(s));
   return RS_OK;
 }
@@ -751,10 +717,10 @@ int rs_resample_mono(rs_engine* e, const void* in_dev, int in_is_pcm16, const in
   if (!e || !in_dev || !len_in_dev || !taps_dev || !out_dev || !len_out_dev) return fail(e, RS_ERR_INVALID_ARG, "rs_resample_mono: bad arguments");
   RS_CUDA(e, cudaSetDevice(e->device));
   Nvtx range("rs::resample_mono");
-  e->cur_stream = static_cast<cudaStream_t>(stream);
   rs::ResampleArgs a{in_dev, in_is_pcm16 != 0, len_in_dev, B, channels, L_in_max, taps_dev, taps_per_phase, up, down, n_pre_remove, pad,
                      out_dev, L_out_row, len_out_dev};
-  RS_K(e, rs::launch_resample_mono(a, static_cast<cudaStream_t>(stream)), 1);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  RS_K(e, s, rs::launch_resample_mono(a, s), 1);
   return RS_OK;
 }
 
@@ -769,8 +735,8 @@ int rs_layernorm(rs_engine* e, const float* x, const float* gamma, const float* 
                  int rows, int d, void* stream) {
   if (!e || !x || !gamma || !beta) return fail(e, RS_ERR_INVALID_ARG, "rs_layernorm: bad arguments");
   RS_CUDA(e, cudaSetDevice(e->device));
-  RS_K(e, rs::launch_layernorm(x, gamma, beta, out_f32, out_bf16, nullptr, nullptr, rows, d, e->cfg.ln_eps,
-                               static_cast<cudaStream_t>(stream)), 1);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  RS_K(e, s, rs::launch_layernorm(x, gamma, beta, out_f32, out_bf16, nullptr, nullptr, rows, d, e->cfg.ln_eps, s), 1);
   return RS_OK;
 }
 
@@ -804,8 +770,8 @@ int rs_debug_decode_cycles(rs_engine* e, int B, int L_max, int U_max, int64_t* o
 
 int rs_enable_kernel_timing(rs_engine* e, int on) {
   if (!e) return RS_ERR_INVALID_ARG;
-  e->ktiming = on != 0;
-  e->k_tag.clear();
+  e->kernel_log.on = on != 0;
+  e->kernel_log.clear();
   return RS_OK;
 }
 
@@ -814,11 +780,10 @@ int rs_kernel_timing(rs_engine* e, char* buf, int buf_bytes) {
   if (!e || !buf || buf_bytes <= 0) return RS_ERR_INVALID_ARG;
   RS_CUDA(e, cudaDeviceSynchronize());
   std::map<std::string, std::pair<int, double>> agg;
-  for (size_t i = 0; i < e->k_tag.size(); ++i) {
-    float t = 0.f;
-    cudaEventElapsedTime(&t, e->k_ev[2 * i], e->k_ev[2 * i + 1]);
-    auto& a = agg[e->k_tag[i]];
-    a.first += 1; a.second += t;
+  const EventLog& log = e->kernel_log;
+  for (size_t i = 0; i < log.entries.size(); ++i) {
+    auto& a = agg[log.entries[i].first];
+    a.first += 1; a.second += log.ms(i);
   }
   std::string out;
   char line[160];
@@ -827,7 +792,7 @@ int rs_kernel_timing(rs_engine* e, char* buf, int buf_bytes) {
     out += line;
   }
   snprintf(buf, static_cast<size_t>(buf_bytes), "%s", out.c_str());
-  e->k_tag.clear();
+  e->kernel_log.clear();
   return RS_OK;
 }
 
@@ -847,25 +812,20 @@ int rs_debug_gemm_cycles(rs_engine* e, int64_t* out64) {
 
 int rs_enable_gemm_timing(rs_engine* e, int on) {
   if (!e) return RS_ERR_INVALID_ARG;
-  e->gemm_timing = on != 0;
-  e->gemm_ev_used = 0;
-  e->gemm_flops = 0.0;
+  e->gemm_log.on = on != 0;
+  e->gemm_log.clear();
   return RS_OK;
 }
 
 int rs_gemm_timing(rs_engine* e, double* ms, double* flops, int64_t* launches) {
   if (!e || !ms || !flops || !launches) return RS_ERR_INVALID_ARG;
-  double total = 0.0;
-  if (e->gemm_ev_used > 0) {
-    RS_CUDA(e, cudaEventSynchronize(e->gemm_ev[e->gemm_ev_used - 1]));
-    for (size_t i = 0; i + 1 < e->gemm_ev_used; i += 2) {
-      float t = 0.f;
-      cudaEventElapsedTime(&t, e->gemm_ev[i], e->gemm_ev[i + 1]);
-      total += t;
-    }
-  }
-  *ms = total; *flops = e->gemm_flops; *launches = static_cast<int64_t>(e->gemm_ev_used / 2);
-  e->gemm_ev_used = 0; e->gemm_flops = 0.0;
+  EventLog& log = e->gemm_log;
+  const size_t n = log.entries.size();
+  if (n > 0) RS_CUDA(e, cudaEventSynchronize(log.ev[2 * n - 1]));
+  double total = 0.0, total_flops = 0.0;
+  for (size_t i = 0; i < n; ++i) { total += log.ms(i); total_flops += log.entries[i].second; }
+  *ms = total; *flops = total_flops; *launches = static_cast<int64_t>(n);
+  log.clear();
   return RS_OK;
 }
 

@@ -36,16 +36,13 @@ struct GemmDev {
   int epilogue;
   float alpha;
   int ldo;              // output (and residual) row stride in elements
-  // optional batching along columns (one launch for all attention heads): batch b reads A columns
-  // [b*a_col_stride, +K), W rows [b*w_row_stride, +N), bias + b*bias_stride, writes columns + b*out_col_stride
-  int n_batch, a_col_stride, w_row_stride, bias_stride, out_col_stride;
   void* out2; int split, ld2;    // RS_EPI_QKV_VT
 };
 template <int BN>
 struct GemmCfg {
   static constexpr int kBBytes = BN * BK * 2;
   static constexpr int kStageBytes = kABytes + kBBytes;
-  static constexpr int kStages = (BN == 256) ? 3 : (BN == 128 ? 5 : 7);
+  static constexpr int kStages = BN == 128 ? 5 : 7;
   static constexpr int kTmemCols = 2 * BN;                       // power of two >= 32
   static constexpr int kSmemBytes = kStages * kStageBytes + 1024 /*align slack*/ + 256 /*barriers*/ + kEpiWarps * (32 * 36 * 4 + 512) /*epilogue staging*/;
 };
@@ -59,12 +56,12 @@ struct GemmCfg {
 constexpr int kStageLd = 36;                                   // floats per staged row (144 B: 16 B-aligned, conflict-free)
 constexpr int kStageBytesPerWarp = 32 * kStageLd * 4 + 512;    // + the bias of the warp's (up to) four chunks of a tile
 
-__device__ __forceinline__ void resid_prefetch(const GemmDev& p, bool on, int tile_row0, int lane, int col0, int bt, float4 (&rr)[8]) {
+__device__ __forceinline__ void resid_prefetch(const GemmDev& p, bool on, int tile_row0, int lane, int col0, float4 (&rr)[8]) {
   if (on) {
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
       const int row = tile_row0 + i * 4 + (lane >> 3);
-      rr[i] = row < p.M ? *reinterpret_cast<const float4*>(p.resid + static_cast<size_t>(row) * p.ldo + bt * p.out_col_stride + col0 + (lane & 7) * 4)
+      rr[i] = row < p.M ? *reinterpret_cast<const float4*>(p.resid + static_cast<size_t>(row) * p.ldo + col0 + (lane & 7) * 4)
                         : make_float4(0.f, 0.f, 0.f, 0.f);
     }
   }
@@ -75,7 +72,7 @@ __device__ __forceinline__ void resid_prefetch(const GemmDev& p, bool on, int ti
 // kResid: the instance may be asked for RS_EPI_RESID_F32 with the residual in rr (otherwise rr is never read).
 template <int EG, bool kResid>
 __device__ __forceinline__ void epilogue_store(const GemmDev& p, const uint32_t (&r)[32], float* stage, int tile_row0, int lane,
-                                               int col0, int bt, const float4 (&rr)[8], const float* bias_s = nullptr) {
+                                               int col0, const float4 (&rr)[8], const float* bias_s = nullptr) {
   float v[32];
 #pragma unroll
   for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
@@ -86,14 +83,13 @@ __device__ __forceinline__ void epilogue_store(const GemmDev& p, const uint32_t 
       v[4 * j] += b.x; v[4 * j + 1] += b.y; v[4 * j + 2] += b.z; v[4 * j + 3] += b.w;
     }
   } else if (p.bias != nullptr) {
-    const float4* b4 = reinterpret_cast<const float4*>(p.bias + bt * p.bias_stride + col0);
+    const float4* b4 = reinterpret_cast<const float4*>(p.bias + col0);
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const float4 b = __ldg(b4 + j);
       v[4 * j] += b.x; v[4 * j + 1] += b.y; v[4 * j + 2] += b.z; v[4 * j + 3] += b.w;
     }
   }
-  const size_t col_off = static_cast<size_t>(bt) * p.out_col_stride;
   uint32_t* stage_u = reinterpret_cast<uint32_t*>(stage);
   int epi = p.epilogue;
   if constexpr (EG == 1) {
@@ -131,7 +127,7 @@ __device__ __forceinline__ void epilogue_store(const GemmDev& p, const uint32_t 
         const int row = tile_row0 + rl;
         const uint4 a = *reinterpret_cast<const uint4*>(stage_u + rl * 20 + cw);
         if (row < p.M)
-          *reinterpret_cast<uint4*>(static_cast<__half*>(p.out) + static_cast<size_t>(row) * p.ldo + col_off + col0 + cw * 2) = a;
+          *reinterpret_cast<uint4*>(static_cast<__half*>(p.out) + static_cast<size_t>(row) * p.ldo + col0 + cw * 2) = a;
       }
       break;
     }
@@ -157,7 +153,7 @@ __device__ __forceinline__ void epilogue_store(const GemmDev& p, const uint32_t 
         const int row = tile_row0 + rl;
         const uint4 a = *reinterpret_cast<const uint4*>(stage_u + rl * 20 + cw);
         if (row < p.M)
-          *reinterpret_cast<uint4*>(static_cast<__nv_bfloat16*>(p.out) + static_cast<size_t>(row) * p.ldo + col_off + col0 + cw * 2) = a;
+          *reinterpret_cast<uint4*>(static_cast<__nv_bfloat16*>(p.out) + static_cast<size_t>(row) * p.ldo + col0 + cw * 2) = a;
       }
       break;
     }
@@ -178,7 +174,7 @@ __device__ __forceinline__ void epilogue_store(const GemmDev& p, const uint32_t 
         const int row = tile_row0 + rl;
         const uint4 a = *reinterpret_cast<const uint4*>(stage_u + rl * 12 + cw);
         if (row < p.M)
-          *reinterpret_cast<uint4*>(static_cast<__nv_bfloat16*>(p.out) + static_cast<size_t>(row) * p.ldo + col_off + col0 / 2 + cw * 2) = a;
+          *reinterpret_cast<uint4*>(static_cast<__nv_bfloat16*>(p.out) + static_cast<size_t>(row) * p.ldo + col0 / 2 + cw * 2) = a;
       }
       break;
     }
@@ -196,7 +192,7 @@ __device__ __forceinline__ void epilogue_store(const GemmDev& p, const uint32_t 
         float4 a = *reinterpret_cast<const float4*>(stage + rl * LD + cw);
         if (add) { a.x += rr[i].x; a.y += rr[i].y; a.z += rr[i].z; a.w += rr[i].w; }
         if (row < p.M)
-          *reinterpret_cast<float4*>(static_cast<float*>(p.out) + static_cast<size_t>(row) * p.ldo + col_off + col0 + cw) = a;
+          *reinterpret_cast<float4*>(static_cast<float*>(p.out) + static_cast<size_t>(row) * p.ldo + col0 + cw) = a;
       }
       break;
     }
@@ -225,8 +221,7 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_const
   const int lane = lane_id();
   const int num_m = (p.M + BM - 1) / BM;
   const int num_n = (p.N + BN - 1) / BN;
-  const int tiles_per_batch = num_m * num_n;
-  const int num_tiles = tiles_per_batch * p.n_batch;
+  const int num_tiles = num_m * num_n;
   const int num_k = p.K / BK;
 
   if (warp == 0 && lane == 0) {
@@ -248,13 +243,12 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_const
     if (lane == 0) {
       int stage = 0; uint32_t phase = 0;
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        const int bt = tile / tiles_per_batch, tl = tile % tiles_per_batch;
-        const int m0 = (tl / num_n) * BM, n0 = (tl % num_n) * BN;
+        const int m0 = (tile / num_n) * BM, n0 = (tile % num_n) * BN;
         for (int kb = 0; kb < num_k; ++kb) {
           mbar_wait(empty_bar(stage), phase ^ 1u);
           mbar_arrive_expect_tx(full_bar(stage), Cfg::kStageBytes);
-          tma_load_2d(smem_a(stage), &tm_a, bt * p.a_col_stride + kb * BK, m0, full_bar(stage));
-          tma_load_2d(smem_b(stage), &tm_b, kb * BK, bt * p.w_row_stride + n0, full_bar(stage));
+          tma_load_2d(smem_a(stage), &tm_a, kb * BK, m0, full_bar(stage));
+          tma_load_2d(smem_b(stage), &tm_b, kb * BK, n0, full_bar(stage));
           if (++stage == Cfg::kStages) { stage = 0; phase ^= 1u; }
         }
       }
@@ -296,13 +290,12 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_const
     for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++it) {
       const int acc = it & 1;
       const uint32_t acc_phase = (it >> 1) & 1u;
-      const int bt = tile / tiles_per_batch, tl = tile % tiles_per_batch;
-      const int m0 = (tl / num_n) * BM, n0 = (tl % num_n) * BN;
+      const int m0 = (tile / num_n) * BM, n0 = (tile % num_n) * BN;
       const int tile_row0 = m0 + q * 32;
       // residual of the first chunk is fetched while the tile's MMAs are still running
       const bool pre = p.epilogue == RS_EPI_RESID_F32;
       float4 rr[8], cur[8];
-      resid_prefetch(p, pre && n0 + half * 32 < p.N, tile_row0, lane, n0 + half * 32, bt, rr);
+      resid_prefetch(p, pre && n0 + half * 32 < p.N, tile_row0, lane, n0 + half * 32, rr);
       mbar_wait(tfull_bar(acc), acc_phase);
       tcgen05_fence_after();
 #pragma unroll 1
@@ -311,11 +304,11 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_const
         if (col0 >= p.N) break;                              // warp-uniform
 #pragma unroll
         for (int j = 0; j < 8; ++j) cur[j] = rr[j];
-        resid_prefetch(p, pre && chunk + 2 < BN / 32 && col0 + 64 < p.N, tile_row0, lane, col0 + 64, bt, rr);
+        resid_prefetch(p, pre && chunk + 2 < BN / 32 && col0 + 64 < p.N, tile_row0, lane, col0 + 64, rr);
         uint32_t r[32];
         tmem_ld_32x32(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * BN + chunk * 32, r);
         tmem_ld_wait();
-        epilogue_store<EG, true>(p, r, stage, tile_row0, lane, col0, bt, cur);
+        epilogue_store<EG, true>(p, r, stage, tile_row0, lane, col0, cur);
       }
       tcgen05_fence_before();
       __syncwarp();
@@ -509,7 +502,7 @@ gemm_bf16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_
         }
       } else {
         [[maybe_unused]] float4 rr[8], cur[8];                                // EG 3 only: the residual, one chunk ahead
-        if constexpr (EG == 3) resid_prefetch(p, true, tile_row0, lane, n0 + half * 32, 0, rr);       // overlaps the tile's MMAs
+        if constexpr (EG == 3) resid_prefetch(p, true, tile_row0, lane, n0 + half * 32, rr);       // overlaps the tile's MMAs
         // the bias of the warp's four chunks -> its shared slot while the MMAs run, read back as broadcasts: with the loads inside
         // the chunk loop every chunk began with an L1 / L2 round trip (same box, three alternating runs: all GEMMs 12.12 ->
         // 11.94 ms per step, N = 4096 3.79 -> 3.62 ms; profiles/r02_ab.md)
@@ -527,12 +520,12 @@ gemm_bf16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_
           if constexpr (EG == 3) {
 #pragma unroll
             for (int j = 0; j < 8; ++j) cur[j] = rr[j];
-            resid_prefetch(p, chunk + 2 < BN / 32, tile_row0, lane, col0 + 64, 0, rr);
+            resid_prefetch(p, chunk + 2 < BN / 32, tile_row0, lane, col0 + 64, rr);
           }
           uint32_t r[32];
           tmem_ld_32x32(t_addr + (chunk - half) * 32, r);
           tmem_ld_wait();
-          epilogue_store<EG, EG == 3>(p, r, stage, tile_row0, lane, col0, 0, cur, bias_s + (chunk >> 1) * 32);
+          epilogue_store<EG, EG == 3>(p, r, stage, tile_row0, lane, col0, cur, bias_s + (chunk >> 1) * 32);
         }
       }
       tcgen05_fence_before();
@@ -607,6 +600,8 @@ static bool make_tmap_f32_chunk(CUtensorMap* m, const void* ptr, uint64_t rows, 
 cudaError_t gemm_debug_cycles(long long* out64) { return cudaMemcpyFromSymbol(out64, g_gemm_prof, sizeof(long long) * 64); }
 
 inline int epilogue_group(int epilogue) { return epilogue == RS_EPI_QKV_VT ? 1 : 0; }
+// output (and residual) row stride: GLU writes one column per value / gate pair
+inline int out_ld(const GemmArgs& g) { return g.epilogue == RS_EPI_BIAS_GLU_BF16 ? g.N / 2 : g.N; }
 
 template <int BN, int EG>
 static cudaError_t launch_bn_eg(const GemmArgs& g, int num_sms, cudaStream_t stream, char* err) {
@@ -618,15 +613,10 @@ static cudaError_t launch_bn_eg(const GemmArgs& g, int num_sms, cudaStream_t str
     attr_once.set();
   }
   CUtensorMap tm_a, tm_b;
-  const int nb = g.n_batch > 0 ? g.n_batch : 1;
-  const int lda = g.lda > 0 ? g.lda : g.K;
-  const int a_cols = nb > 1 ? (nb - 1) * g.a_col_stride + g.K : g.K;
-  const int w_rows = nb > 1 ? (nb - 1) * g.w_row_stride + g.N : g.N;
-  const int ldo = g.ldo > 0 ? g.ldo : (g.epilogue == RS_EPI_BIAS_GLU_BF16 ? g.N / 2 : g.N);
-  if (!make_tmap_bf16(&tm_a, g.a, g.M, a_cols, lda, BM, err)) return cudaErrorInvalidValue;
-  if (!make_tmap_bf16(&tm_b, g.w, w_rows, g.K, g.K, BN, err)) return cudaErrorInvalidValue;
-  GemmDev p{g.bias, g.resid, g.out, g.M, g.N, g.K, g.epilogue, g.alpha, ldo, nb, g.a_col_stride, g.w_row_stride, g.bias_stride, g.out_col_stride, g.out2, g.split, g.ld2};
-  const int tiles = ((g.M + BM - 1) / BM) * ((g.N + BN - 1) / BN) * nb;
+  if (!make_tmap_bf16(&tm_a, g.a, g.M, g.K, g.K, BM, err)) return cudaErrorInvalidValue;
+  if (!make_tmap_bf16(&tm_b, g.w, g.N, g.K, g.K, BN, err)) return cudaErrorInvalidValue;
+  const GemmDev p{g.bias, g.resid, g.out, g.M, g.N, g.K, g.epilogue, g.alpha, out_ld(g), g.out2, g.split, g.ld2};
+  const int tiles = ((g.M + BM - 1) / BM) * ((g.N + BN - 1) / BN);
   const int grid = tiles < num_sms ? tiles : num_sms;
   gemm_bf16_tn_kernel<BN, EG><<<grid, kGemmThreads, Cfg::kSmemBytes, stream>>>(tm_a, tm_b, p);
   cudaError_t e = cudaGetLastError();
@@ -652,13 +642,11 @@ static cudaError_t launch_2cta_eg(const GemmArgs& g, int num_sms, cudaStream_t s
     attr_once.set();
   }
   CUtensorMap tm_a, tm_b, tm_o;
-  const int lda = g.lda > 0 ? g.lda : g.K;
-  const int ldo = g.ldo > 0 ? g.ldo : (g.epilogue == RS_EPI_BIAS_GLU_BF16 ? g.N / 2 : g.N);
-  if (!make_tmap_bf16(&tm_a, g.a, g.M, g.K, lda, BM, err)) return cudaErrorInvalidValue;
+  if (!make_tmap_bf16(&tm_a, g.a, g.M, g.K, g.K, BM, err)) return cudaErrorInvalidValue;
   if (!make_tmap_bf16(&tm_b, g.w, g.N, g.K, g.K, BN / 2, err)) return cudaErrorInvalidValue;
-  if (EG == 2) { if (!make_tmap_f32_chunk(&tm_o, g.out, g.M, g.N, ldo, err)) return cudaErrorInvalidValue; }
+  if (EG == 2) { if (!make_tmap_f32_chunk(&tm_o, g.out, g.M, g.N, out_ld(g), err)) return cudaErrorInvalidValue; }
   else memset(&tm_o, 0, sizeof(tm_o));
-  const GemmDev p{g.bias, g.resid, g.out, g.M, g.N, g.K, g.epilogue, g.alpha, ldo, 1, 0, 0, 0, 0, g.out2, g.split, g.ld2};
+  const GemmDev p{g.bias, g.resid, g.out, g.M, g.N, g.K, g.epilogue, g.alpha, out_ld(g), g.out2, g.split, g.ld2};
   const int tiles = ((g.M + 2 * BM - 1) / (2 * BM)) * (g.N / BN);
   int clusters = num_sms / 2;
   if (tiles < clusters) clusters = tiles;
@@ -671,8 +659,7 @@ static cudaError_t launch_2cta_eg(const GemmArgs& g, int num_sms, cudaStream_t s
 template <int BN>
 static cudaError_t launch_2cta(const GemmArgs& g, int num_sms, cudaStream_t stream, char* err) {
   // residual added in place: handed to the memory system as a TMA reduce-add (see Gemm2Cfg)
-  const int ldo = g.ldo > 0 ? g.ldo : g.N;
-  if (g.epilogue == RS_EPI_RESID_F32 && g.resid == g.out && ldo % 4 == 0) return launch_2cta_eg<BN, 2>(g, num_sms, stream, err);
+  if (g.epilogue == RS_EPI_RESID_F32 && g.resid == g.out) return launch_2cta_eg<BN, 2>(g, num_sms, stream, err);
   if (g.epilogue == RS_EPI_RESID_F32) return launch_2cta_eg<BN, 3>(g, num_sms, stream, err);   // residual from another buffer: read into registers
   switch (epilogue_group(g.epilogue)) {
     case 1: return launch_2cta_eg<BN, 1>(g, num_sms, stream, err);
@@ -690,16 +677,14 @@ cudaError_t launch_gemm(const GemmArgs& g, int num_sms, cudaStream_t stream, cha
     return cudaErrorInvalidValue;
   }
   if (g.epilogue == RS_EPI_RESID_F32 && g.resid == nullptr) { snprintf(err, 256, "gemm: residual epilogue without resid"); return cudaErrorInvalidValue; }
-  if (g.epilogue == RS_EPI_QKV_VT && (g.out2 == nullptr || g.split % 32 || g.ld2 % 8 || g.M % 8 || g.ld2 < g.M || g.n_batch > 1)) {
+  if (g.epilogue == RS_EPI_QKV_VT && (g.out2 == nullptr || g.split % 32 || g.ld2 % 8 || g.M % 8 || g.ld2 < g.M)) {
     snprintf(err, 256, "gemm: RS_EPI_QKV_VT needs out2, split %% 32 == 0, ld2 %% 8 == 0, M %% 8 == 0, ld2 >= M");
     return cudaErrorInvalidValue;
   }
   // kernel choice depends on N only (never on M): a row's result must not depend on the batch it sits in
-  if (g.n_batch <= 1 && g.N % 256 == 0)                       // 2-CTA pairs (cta_group::2), 256 x 256 tiles
-    return launch_2cta<256>(g, num_sms, stream, err);
-  // 1-CTA kernel: the column-batched launch and N not divisible by 256; the widest tile that divides N
-  if (g.N >= 256 && g.N % 256 == 0) return launch_bn<256>(g, num_sms, stream, err);
-  if (g.N >= 128 && g.N % 128 == 0) return launch_bn<128>(g, num_sms, stream, err);
+  if (g.N % 256 == 0) return launch_2cta<256>(g, num_sms, stream, err);   // 2-CTA pairs (cta_group::2), 256 x 256 tiles
+  // 1-CTA kernel for N not divisible by 256: the widest tile that divides N
+  if (g.N % 128 == 0) return launch_bn<128>(g, num_sms, stream, err);
   return launch_bn<64>(g, num_sms, stream, err);
 }
 

@@ -14,9 +14,6 @@ struct GemmArgs {
   int M, N, K;
   int epilogue;        // rs_epilogue
   float alpha;
-  // optional: A row stride (elements, default K), output row stride (default N), column batching
-  int lda = 0, ldo = 0;
-  int n_batch = 1, a_col_stride = 0, w_row_stride = 0, bias_stride = 0, out_col_stride = 0;
   // RS_EPI_QKV_VT: columns >= split go, transposed, to out2 (bf16 [N - split, ld2]; ld2 >= M rounded up to 256)
   void* out2 = nullptr; int split = 0, ld2 = 0;
 };

@@ -44,13 +44,44 @@ class RsTensor(C.Structure):
 _DTYPES = {torch.float32: 0, torch.bfloat16: 1, torch.int32: 2}
 _lib = None
 
-EXPORTS = [
-    "rs_engine_create", "rs_engine_destroy", "rs_last_error", "rs_workspace_bytes", "rs_set_workspace",
-    "rs_mel_frames", "rs_enc_frames", "rs_mel_valid", "rs_enc_valid", "rs_logmel", "rs_encode", "rs_rnnt_greedy", "rs_transcribe_device",
-    "rs_transcribe_batch", "rs_transcribe_device_pcm16", "rs_transcribe_batch_pcm16", "rs_resample_mono", "rs_rnnt_alsd", "rs_gemm_bf16", "rs_layernorm", "rs_launch_count", "rs_enable_stage_timing",
-    "rs_stage_times_ms", "rs_enable_gemm_timing", "rs_gemm_timing", "rs_debug_decode_cycles",
-    "rs_enable_kernel_timing", "rs_kernel_timing", "rs_debug_attention_cycles", "rs_debug_gemm_cycles", "rs_stage_rows",
-]
+_vp, _ip, _i64, _f32, _f64 = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_double
+_P = C.POINTER
+_XCRIBE = [_vp, _vp, _vp, _ip, _ip, _vp, _vp, _vp, _ip, _vp]       # the four rs_transcribe_* entry points
+# ctypes signature of every C-ABI entry point (include/rs_engine.h): name -> (restype, argtypes)
+SIGNATURES = {
+    "rs_engine_create": (_ip, [_P(RsModelConfig), _P(RsTensor), _ip, _ip, _P(_vp)]),
+    "rs_engine_destroy": (None, [_vp]),
+    "rs_last_error": (C.c_char_p, [_vp]),
+    "rs_workspace_bytes": (_ip, [_vp, _ip, _ip, _P(C.c_size_t)]),
+    "rs_set_workspace": (_ip, [_vp, _vp, C.c_size_t]),
+    "rs_mel_frames": (_ip, [_vp, _ip]),
+    "rs_enc_frames": (_ip, [_vp, _ip]),
+    "rs_mel_valid": (_ip, [_vp, _ip]),
+    "rs_enc_valid": (_ip, [_vp, _ip]),
+    "rs_logmel": (_ip, [_vp, _vp, _vp, _ip, _ip, _vp, _vp, _vp]),
+    "rs_encode": (_ip, [_vp, _vp, _vp, _ip, _ip, _vp, _vp, _ip, _vp]),
+    "rs_rnnt_greedy": (_ip, [_vp, _vp, _vp, _ip, _ip, _vp, _vp, _vp, _ip, _vp]),
+    "rs_transcribe_device": (_ip, _XCRIBE),
+    "rs_transcribe_batch": (_ip, _XCRIBE),
+    "rs_transcribe_device_pcm16": (_ip, _XCRIBE),
+    "rs_transcribe_batch_pcm16": (_ip, _XCRIBE),
+    "rs_resample_mono": (_ip, [_vp, _vp, _ip, _vp, _ip, _ip, _ip, _vp, _ip, _ip, _ip, _ip, _ip, _vp, _ip, _vp, _vp]),
+    "rs_rnnt_alsd": (_ip, [_vp, _vp, _vp, _ip, _ip, _ip, _f32, _ip, _ip, _vp, _vp, _vp, _vp, _ip, _vp]),
+    "rs_gemm_bf16": (_ip, [_vp, _vp, _vp, _vp, _vp, _vp, _ip, _ip, _ip, _ip, _f32, _vp]),
+    "rs_layernorm": (_ip, [_vp, _vp, _vp, _vp, _vp, _vp, _ip, _ip, _vp]),
+    "rs_launch_count": (_i64, [_vp]),
+    "rs_enable_stage_timing": (_ip, [_vp, _ip]),
+    "rs_stage_times_ms": (_ip, [_vp, _P(_f32)]),
+    "rs_enable_gemm_timing": (_ip, [_vp, _ip]),
+    "rs_gemm_timing": (_ip, [_vp, _P(_f64), _P(_f64), _P(_i64)]),
+    "rs_debug_decode_cycles": (_ip, [_vp, _ip, _ip, _ip, _P(_i64)]),
+    "rs_enable_kernel_timing": (_ip, [_vp, _ip]),
+    "rs_kernel_timing": (_ip, [_vp, C.c_char_p, _ip]),
+    "rs_debug_attention_cycles": (_ip, [_vp, _P(_i64)]),
+    "rs_debug_gemm_cycles": (_ip, [_vp, _P(_i64)]),
+    "rs_stage_rows": (_ip, [_vp, _i64, _P(_vp), _P(_i64), _P(C.c_int32), _ip, _ip, _i64, _ip]),
+}
+EXPORTS = list(SIGNATURES)
 
 
 def load_library(build_if_missing: bool = True) -> C.CDLL:
@@ -58,60 +89,15 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     global _lib
     if _lib is not None:
         return _lib
-    path = _LIB_PATH
     if not os.path.exists(_LIB_PATH):
         if not build_if_missing:
             raise FileNotFoundError(_LIB_PATH)
         from .build import build
         build()
-    lib = C.CDLL(path)
-    vp, ip, i32p, f32p = C.c_void_p, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_float)
-    lib.rs_engine_create.argtypes = [C.POINTER(RsModelConfig), C.POINTER(RsTensor), ip, ip, C.POINTER(vp)]
-    lib.rs_engine_create.restype = ip
-    lib.rs_engine_destroy.argtypes = [vp]
-    lib.rs_engine_destroy.restype = None
-    lib.rs_last_error.argtypes = [vp]
-    lib.rs_last_error.restype = C.c_char_p
-    lib.rs_workspace_bytes.argtypes = [vp, ip, ip, C.POINTER(C.c_size_t)]
-    lib.rs_set_workspace.argtypes = [vp, vp, C.c_size_t]
-    lib.rs_mel_frames.argtypes = [vp, ip]
-    lib.rs_enc_frames.argtypes = [vp, ip]
-    lib.rs_mel_valid.argtypes = [vp, ip]
-    lib.rs_enc_valid.argtypes = [vp, ip]
-    lib.rs_logmel.argtypes = [vp, vp, vp, ip, ip, vp, vp, vp]
-    lib.rs_encode.argtypes = [vp, vp, vp, ip, ip, vp, vp, ip, vp]
-    lib.rs_rnnt_greedy.argtypes = [vp, vp, vp, ip, ip, vp, vp, vp, ip, vp]
-    lib.rs_transcribe_device.argtypes = [vp, vp, vp, ip, ip, vp, vp, vp, ip, vp]
-    lib.rs_transcribe_batch.argtypes = [vp, vp, vp, ip, ip, vp, vp, vp, ip, vp]
-    lib.rs_transcribe_device_pcm16.argtypes = [vp, vp, vp, ip, ip, vp, vp, vp, ip, vp]
-    lib.rs_transcribe_batch_pcm16.argtypes = [vp, vp, vp, ip, ip, vp, vp, vp, ip, vp]
-    lib.rs_rnnt_alsd.argtypes = [vp, vp, vp, ip, ip, ip, C.c_float, ip, ip, vp, vp, vp, vp, ip, vp]
-    lib.rs_rnnt_alsd.restype = ip
-    lib.rs_resample_mono.argtypes = [vp, vp, ip, vp, ip, ip, ip, vp, ip, ip, ip, ip, ip, vp, ip, vp, vp]
-    lib.rs_resample_mono.restype = ip
-    lib.rs_gemm_bf16.argtypes = [vp, vp, vp, vp, vp, vp, ip, ip, ip, ip, C.c_float, vp]
-    lib.rs_layernorm.argtypes = [vp, vp, vp, vp, vp, vp, ip, ip, vp]
-    lib.rs_launch_count.argtypes = [vp]
-    lib.rs_launch_count.restype = C.c_int64
-    lib.rs_enable_stage_timing.argtypes = [vp, ip]
-    lib.rs_stage_times_ms.argtypes = [vp, f32p]
-    lib.rs_debug_decode_cycles.argtypes = [vp, ip, ip, ip, C.POINTER(C.c_int64)]
-    lib.rs_debug_decode_cycles.restype = ip
-    lib.rs_debug_gemm_cycles.argtypes = [vp, C.POINTER(C.c_int64)]
-    lib.rs_debug_gemm_cycles.restype = ip
-    lib.rs_stage_rows.argtypes = [vp, C.c_int64, C.POINTER(vp), C.POINTER(C.c_int64), i32p, ip, ip, C.c_int64, ip]
-    lib.rs_stage_rows.restype = ip
-    lib.rs_enable_kernel_timing.argtypes = [vp, ip]
-    lib.rs_enable_kernel_timing.restype = ip
-    lib.rs_kernel_timing.argtypes = [vp, C.c_char_p, ip]
-    lib.rs_kernel_timing.restype = ip
-    lib.rs_enable_gemm_timing.argtypes = [vp, ip]
-    lib.rs_gemm_timing.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_int64)]
-    for fn in ("rs_workspace_bytes", "rs_set_workspace", "rs_mel_frames", "rs_enc_frames", "rs_mel_valid", "rs_enc_valid", "rs_logmel", "rs_encode",
-               "rs_rnnt_greedy", "rs_transcribe_device", "rs_transcribe_batch", "rs_transcribe_device_pcm16", "rs_transcribe_batch_pcm16",
-               "rs_gemm_bf16", "rs_layernorm",
-               "rs_enable_stage_timing", "rs_stage_times_ms", "rs_enable_gemm_timing", "rs_gemm_timing"):
-        getattr(lib, fn).restype = ip
+    lib = C.CDLL(_LIB_PATH)
+    for name, (restype, argtypes) in SIGNATURES.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = lib
     return lib
 
@@ -164,7 +150,7 @@ def pack_weights(sd: StateDict, cfg: ModelConfig) -> Dict[str, torch.Tensor]:
         n_rel_pad = (cfg.n_rel + 31) // 32 * 32
         pos_h = torch.zeros(H, n_rel_pad, dk)
         pos_h[:, : cfg.n_rel] = pos.view(cfg.n_rel, H, dk).permute(1, 0, 2)
-        out[o + "att.pos"] = bf(pos_h)                                                 # B operand of the batched BD GEMM
+        out[o + "att.pos"] = bf(pos_h)                                                 # operand of the attention kernel's positional UMMA
         # (q + v).p = (q + u).p + (v - u).p: the second term is input independent -> the GEMM's bias
         out[o + "att.bdbias"] = f32((out[o + "att.pos"].float() * (sd[a + "pos_bias_v"] - sd[a + "pos_bias_u"])[:, None, :]).sum(-1).reshape(-1))
         out[o + "att.u"] = f32(sd[a + "pos_bias_u"].reshape(-1))
@@ -463,7 +449,6 @@ class Engine:
     def attention_cycles(self):
         """clock64 stamps of CTA (1,0,0) of the last tensor-core attention launch, relative to its first stamp."""
         out = (C.c_int64 * 16)()
-        self.lib.rs_debug_attention_cycles.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
         self._check(self.lib.rs_debug_attention_cycles(self.h, out), "rs_debug_attention_cycles")
         v = list(out)
         names = ["start", "tma_issue", "qk_landed", "s_issued", "pv_wait", "pv_issued", "dealloc", "_",
