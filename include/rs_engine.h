@@ -149,6 +149,18 @@ int rs_rnnt_alsd(rs_engine* e, const float* enc_dev, const int32_t* enc_len_dev,
                  float u_max_ratio, int score_norm, int recombine_returns_input, int32_t* y_dev, int32_t* step_dev,
                  int32_t* n_dev, double* score_dev, int U_cap, void* stream);
 
+/* RNN-T forced alignment of given token sequences: enc f32[B,T_max,d_model] + enc_len, targets i32[B,U_max] (ids in
+ * [0, vocab_size)) + tgt_len i32[B] -> frames i32[B,U_max] (emitting encoder frame of each token on the Viterbi path),
+ * tok_logp f32[B,U_max], viterbi f64[B], loglik f64[B] (forward sum over all alignments = -RNN-T loss),
+ * lattice f32[B,T_max,U_max+1,2] (nullable: log p(blank), log p(next target) per node; other entries unspecified).
+ * Entries of frames / tok_logp at or beyond tgt_len[b] are -1 / 0.  enc_len[b] in [1, T_max], tgt_len[b] in [0, U_max],
+ * U_max >= 1; a violated range, or a target outside [0, vocab_size), returns RS_ERR_INVALID_ARG before any computation.
+ * Needs the "alsd.*" weight tensors (RS_ERR_UNSUPPORTED without them).  Synchronises before returning. */
+int rs_rnnt_align(rs_engine* e, const float* enc_dev, const int32_t* enc_len_dev, int B, int T_max,
+                  const int32_t* targets_dev, const int32_t* tgt_len_dev, int U_max,
+                  int32_t* frames_dev, float* tok_logp_dev, double* viterbi_dev, double* loglik_dev,
+                  float* lattice_dev, void* stream);
+
 /* norm_audio on the device (pkg/nemo-asr/src/audio.py:54-68: resample to 16 kHz, then average the channels) fused with
  * transcribe()'s padding (audio.py:70-83): in [B, channels, L_in_max] f32 or int16 PCM at the native rate ->
  * out f32 [B, L_out_row], row b = pad zeros | resampled mono utterance | zeros, len_out[b] = resampled length + 2 pad;

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "build")
 LIB = os.path.join(HERE, "librs_engine.so")
-SOURCES = ["gemm_tcgen05.cu", "logmel.cu", "subsample.cu", "elementwise.cu", "resample.cu", "attention_tc.cu", "decode_spec.cu", "decode_alsd.cu", "host_staging.cu", "engine.cu"]
+SOURCES = ["gemm_tcgen05.cu", "logmel.cu", "subsample.cu", "elementwise.cu", "resample.cu", "attention_tc.cu", "decode_spec.cu", "decode_alsd.cu", "align.cu", "host_staging.cu", "engine.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 FLAGS += os.environ.get("RS_BUILD_FLAGS", "").split()        # build-time only, e.g. -DRS_PROF for scripts/diag_gemm_timeline.py

@@ -27,20 +27,13 @@
 #include "alsd.h"
 #include "common.cuh"
 #include "kernels.h"
+#include "rnnt_cell.cuh"
 
 namespace rs {
 
 namespace {
 
 constexpr int kMaxBeam = 8;
-
-// x -> three bf16 values with hi + mid + lo == x to 24 mantissa bits
-__device__ __forceinline__ void split3(float x, __nv_bfloat16& hi, __nv_bfloat16& mid, __nv_bfloat16& lo) {
-  hi = __float2bfloat16_rn(x);
-  const float r1 = x - __bfloat162float(hi);
-  mid = __float2bfloat16_rn(r1);
-  lo = __float2bfloat16_rn(r1 - __bfloat162float(mid));
-}
 
 // ---------------------------------------------------------------------------------------------- joint rows
 // grid (B * beam), block 128.  Row r = b * beam + k.  Dead rows (hypothesis absent, or past the last frame) are zero-filled:
@@ -268,10 +261,7 @@ alsd_cell_kernel(const AlsdState st, const float* __restrict__ gates, int Hp, __
   for (int j = threadIdx.x; j < Hp; j += blockDim.x) {
     float h2 = 0.f, c2 = 0.f;
     if (ext) {
-      const float ig = sigmoidf_accurate(g[j]), fg = sigmoidf_accurate(g[Hp + j]);
-      const float cg = tanhf(g[2 * Hp + j]), og = sigmoidf_accurate(g[3 * Hp + j]);
-      c2 = fg * st.c[pr * Hp + j] + ig * cg;
-      h2 = og * tanhf(c2);
+      lstm_cell(g[j], g[Hp + j], g[2 * Hp + j], g[3 * Hp + j], st.c[pr * Hp + j], h2, c2);
     } else if (live) {
       h2 = st.h[pr * Hp + j]; c2 = st.c[pr * Hp + j];
     }

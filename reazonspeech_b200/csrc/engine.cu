@@ -15,6 +15,7 @@
 #include <vector>
 
 #include "../../include/rs_engine.h"
+#include "align.h"
 #include "alsd.h"
 #include "kernels.h"
 #include "logmel.h"
@@ -93,6 +94,8 @@ struct rs_engine {
   void* alsd_ws = nullptr;
   size_t alsd_ws_bytes = 0;
   int* alsd_done_host = nullptr;
+  void* align_ws = nullptr;             // forced alignment (align.cu): engine-owned, grown on demand
+  size_t align_ws_bytes = 0;
   unsigned int* lm_tickets = nullptr;   // per-utterance CTA tickets of the log-mel statistics (engine-owned, kept zero between launches)
   static constexpr int kMaxBatch = 1 << 16;
   struct { const float *c0w, *c0b, *d1w, *d1b, *p1b, *d2w, *d2b, *p2b, *ob; const void *p1w, *p2w, *ow; } sub;
@@ -557,6 +560,7 @@ void rs_engine_destroy(rs_engine* e) {
   cudaFree(e->lm_tickets);
   cudaFree(e->alsd_ws);
   if (e->alsd_done_host) cudaFreeHost(e->alsd_done_host);
+  cudaFree(e->align_ws);
   delete e;
 }
 
@@ -707,6 +711,96 @@ int rs_rnnt_alsd(rs_engine* e, const float* enc, const int32_t* enc_len, int B, 
     }
   }
   RS_K(e, s, rs::alsd_launch_output(st, B, blank, y_dev, step_dev, n_dev, score_dev, U_cap, s), 1);
+  RS_CUDA(e, cudaStreamSynchronize(s));
+  return RS_OK;
+}
+
+// RNN-T forced alignment of given token sequences (align.cu; semantics: oracle/align_restated.py).  The lengths are read back
+// once to lay out the compact node list (utterance b: T_b * (U_b + 1) nodes); the lattice is evaluated in chunks of
+// kAlignChunkRows nodes so that the bf16 A planes stay bounded.  Synchronises.
+int rs_rnnt_align(rs_engine* e, const float* enc, const int32_t* enc_len, int B, int T_max, const int32_t* targets,
+                  const int32_t* tgt_len, int U_max, int32_t* frames, float* tok_logp, double* viterbi, double* loglik, float* lattice,
+                  void* stream) {
+  if (!e || !enc || !enc_len || !targets || !tgt_len || !frames || !tok_logp || !viterbi || !loglik || B <= 0 || T_max <= 0 || U_max <= 0)
+    return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: bad arguments");
+  if (B > rs_engine::kMaxBatch) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: batch of %d utterances exceeds the engine limit of %d", B, rs_engine::kMaxBatch);
+  if (e->alsd.out_w3 == nullptr)
+    return fail(e, RS_ERR_UNSUPPORTED, "rs_rnnt_align: the engine was created without the aligner weight tensors (alsd.*)");
+  RS_CUDA(e, cudaSetDevice(e->device));
+  Nvtx range("rs::rnnt_align");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const rs_model_config& c = e->cfg;
+  const int Hj = c.joint_hidden, Hp = c.pred_hidden, d = c.d_model, V = c.vocab_size, n_pad = e->alsd.n_pad;
+  std::vector<int32_t> T(B), U(B);
+  RS_CUDA(e, cudaMemcpyAsync(T.data(), enc_len, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, s));
+  RS_CUDA(e, cudaMemcpyAsync(U.data(), tgt_len, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, s));
+  RS_CUDA(e, cudaStreamSynchronize(s));
+  std::vector<int64_t> offs(B + 1, 0);
+  int U_top = 0;
+  for (int b = 0; b < B; ++b) {
+    if (T[b] < 1 || T[b] > T_max) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: enc_len[%d] = %d outside [1, T_max = %d]", b, T[b], T_max);
+    if (U[b] < 0 || U[b] > U_max) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: tgt_len[%d] = %d outside [0, U_max = %d]", b, U[b], U_max);
+    offs[b + 1] = offs[b] + static_cast<int64_t>(T[b]) * (U[b] + 1);
+    U_top = std::max(U_top, U[b]);
+  }
+  const int U1 = U_top + 1;                                // predictor states h_0 .. h_U per utterance
+  if (rs::align_dp_smem_bytes(U1) > 227 * 1024)
+    return fail(e, RS_ERR_UNSUPPORTED, "rs_rnnt_align: %d targets in one utterance exceed what the DP kernel holds in shared memory (%d)",
+                U_top, static_cast<int>(227 * 1024 / rs::align_dp_smem_bytes(1)) - 1);
+  const int64_t total = offs[B];
+  const int chunk = static_cast<int>(std::min<int64_t>(total, rs::kAlignChunkRows));
+  const int M = B * T_max;
+  // ---- workspace
+  Arena a;
+  const size_t o_flag = a.take(256), o_offs = a.take(static_cast<size_t>(B + 1) * 8);
+  const size_t o_xn = a.take(static_cast<size_t>(M) * d * 2), o_encp = a.take(static_cast<size_t>(M) * Hj * 4);
+  const size_t o_in = a.take(static_cast<size_t>(B) * 6 * Hp * 2), o_gates = a.take(static_cast<size_t>(B) * 4 * Hp * 4);
+  const size_t o_c = a.take(static_cast<size_t>(B) * Hp * 4), o_hp = a.take(static_cast<size_t>(B) * U1 * 3 * Hp * 2);
+  const size_t o_g = a.take(static_cast<size_t>(B) * U1 * Hj * 4);
+  const size_t o_planes = a.take(static_cast<size_t>(chunk) * 3 * Hj * 2), o_tcol = a.take(static_cast<size_t>(chunk) * 4);
+  const size_t o_lp = a.take(static_cast<size_t>(total) * 8), o_bp = a.take(static_cast<size_t>(total));
+  if (a.off > e->align_ws_bytes) {
+    RS_CUDA(e, cudaStreamSynchronize(s));
+    cudaFree(e->align_ws); e->align_ws = nullptr; e->align_ws_bytes = 0;
+    RS_CUDA(e, cudaMalloc(&e->align_ws, a.off));
+    e->align_ws_bytes = a.off;
+  }
+  char* ws = static_cast<char*>(e->align_ws);
+  int* flag = reinterpret_cast<int*>(ws + o_flag);
+  const int64_t* offs_dev = reinterpret_cast<const int64_t*>(ws + o_offs);
+  float* encp = reinterpret_cast<float*>(ws + o_encp); float* gates = reinterpret_cast<float*>(ws + o_gates);
+  float* g = reinterpret_cast<float*>(ws + o_g); float2* lp = reinterpret_cast<float2*>(ws + o_lp);
+  // ---- targets outside [0, V) are reported before any kernel indexes a table with them
+  RS_CUDA(e, cudaMemsetAsync(flag, 0, 4, s));
+  RS_K(e, s, rs::align_check(targets, tgt_len, B, U_max, V, flag, s), 1);
+  int bad = 0;
+  RS_CUDA(e, cudaMemcpyAsync(&bad, flag, 4, cudaMemcpyDeviceToHost, s));
+  RS_CUDA(e, cudaStreamSynchronize(s));
+  if (bad) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: a target id lies outside [0, vocab_size = %d)", V);
+  RS_CUDA(e, cudaMemcpyAsync(ws + o_offs, offs.data(), static_cast<size_t>(B + 1) * 8, cudaMemcpyHostToDevice, s));
+  // ---- joint.enc over every frame (as in the greedy path)
+  RS_K(e, s, rs::launch_f32_to_bf16(enc, ws + o_xn, static_cast<int64_t>(M) * d, s), 1);
+  RS_TRY(gemm(e, ws + o_xn, e->dec.enc_w, e->dec.enc_b, nullptr, encp, M, Hj, d, RS_EPI_BIAS_F32, 1.f, s));
+  // ---- teacher-forced predictor: step 0 consumes the blank (zero input, zero state), step k the target y_k
+  RS_CUDA(e, cudaMemsetAsync(ws + o_in, 0, static_cast<size_t>(B) * 6 * Hp * 2, s));
+  for (int k = 0; k <= U_top; ++k) {
+    RS_TRY(gemm(e, ws + o_in, e->alsd.lstm_w3, e->dec.lstm_b, nullptr, gates, B, 4 * Hp, 6 * Hp, RS_EPI_BIAS_F32, 1.f, s));
+    RS_K(e, s, rs::align_pred(gates, reinterpret_cast<float*>(ws + o_c), targets, tgt_len, B, U_max, U1, k, e->dec.embed, Hp,
+                              ws + o_in, ws + o_hp, s), 1);
+  }
+  RS_TRY(gemm(e, ws + o_hp, e->alsd.pred_w3, e->dec.pred_b, nullptr, g, B * U1, Hj, 3 * Hp, RS_EPI_BIAS_F32, 1.f, s));
+  // ---- lattice, chunk by chunk
+  for (int64_t r0 = 0; r0 < total; r0 += chunk) {
+    const int n = static_cast<int>(std::min<int64_t>(chunk, total - r0));
+    RS_K(e, s, rs::align_rows(encp, g, offs_dev, tgt_len, targets, B, T_max, U1, U_max, Hj, r0, n, ws + o_planes,
+                              reinterpret_cast<int32_t*>(ws + o_tcol), s), 1);
+    RS_TRY(launch(e, s, "rs::align_lattice", 1, 0.0, [&](char* msg) {
+      return rs::align_lattice(ws + o_planes, e->alsd.out_w3, e->alsd.out_b, reinterpret_cast<const int32_t*>(ws + o_tcol), lp + r0, n,
+                               n_pad, Hj, V, e->num_sms, s, msg);
+    }));
+  }
+  RS_K(e, s, rs::align_dp(lp, offs_dev, enc_len, tgt_len, B, T_max, U_max, U1, reinterpret_cast<uint8_t*>(ws + o_bp), frames, tok_logp,
+                          viterbi, loglik, lattice, s), 1);
   RS_CUDA(e, cudaStreamSynchronize(s));
   return RS_OK;
 }

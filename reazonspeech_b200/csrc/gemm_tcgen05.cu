@@ -568,7 +568,7 @@ static EncodeTiledFn get_encode_fn() {
 }
 
 // bf16 row-major [rows, cols] -> 2-D map with a (box_rows x 64) box and 128B swizzle.
-static bool make_tmap_bf16(CUtensorMap* m, const void* ptr, uint64_t rows, uint64_t cols, uint64_t ld, uint32_t box_rows, char* err) {
+bool make_tmap_bf16(CUtensorMap* m, const void* ptr, uint64_t rows, uint64_t cols, uint64_t ld, uint32_t box_rows, char* err) {
   EncodeTiledFn fn = get_encode_fn();
   if (fn == nullptr) { snprintf(err, 256, "cuTensorMapEncodeTiled entry point unavailable"); return false; }
   cuuint64_t dims[2] = {cols, rows};

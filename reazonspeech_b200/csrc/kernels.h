@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+struct CUtensorMap_st;
+
 namespace rs {
 
 struct GemmArgs {
@@ -20,6 +22,9 @@ struct GemmArgs {
 
 // Returns cudaSuccess or the failing CUDA error; err (>=256 B) receives a description.
 cudaError_t launch_gemm(const GemmArgs& g, int num_sms, cudaStream_t stream, char* err);
+// TMA descriptor of a bf16 row-major [rows, cols] operand (row pitch ld elements): (box_rows x 64) boxes, 128B swizzle,
+// out-of-range rows zero-filled.  (CUtensorMap_st is cuda.h's CUtensorMap, named here without the driver API include.)
+bool make_tmap_bf16(::CUtensorMap_st* m, const void* ptr, uint64_t rows, uint64_t cols, uint64_t ld, uint32_t box_rows, char* err);
 cudaError_t gemm_debug_cycles(long long* out64);   // timeline of the last 2-CTA launch (see g_gemm_prof)
 
 cudaError_t launch_layernorm(const float* x, const float* gamma, const float* beta, float* out_f32,

@@ -67,6 +67,7 @@ SIGNATURES = {
     "rs_transcribe_batch_pcm16": (_ip, _XCRIBE),
     "rs_resample_mono": (_ip, [_vp, _vp, _ip, _vp, _ip, _ip, _ip, _vp, _ip, _ip, _ip, _ip, _ip, _vp, _ip, _vp, _vp]),
     "rs_rnnt_alsd": (_ip, [_vp, _vp, _vp, _ip, _ip, _ip, _f32, _ip, _ip, _vp, _vp, _vp, _vp, _ip, _vp]),
+    "rs_rnnt_align": (_ip, [_vp, _vp, _vp, _ip, _ip, _vp, _vp, _ip, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rs_gemm_bf16": (_ip, [_vp, _vp, _vp, _vp, _vp, _vp, _ip, _ip, _ip, _ip, _f32, _vp]),
     "rs_layernorm": (_ip, [_vp, _vp, _vp, _vp, _vp, _vp, _ip, _ip, _vp]),
     "rs_launch_count": (_i64, [_vp]),
@@ -379,6 +380,26 @@ class Engine:
                                           int(recombine_returns_input), y.data_ptr(), steps.data_ptr(), n.data_ptr(), score.data_ptr(), U,
                                           self._stream()), "rs_rnnt_alsd")
         return y, steps, n, score
+
+    def align(self, enc: torch.Tensor, enc_len: torch.Tensor, targets: torch.Tensor, tgt_len: torch.Tensor, lattice: bool = False):
+        """RNN-T forced alignment of the given token sequences (needs the ``alsd.*`` tensors: ``Engine(..., alsd=True)``).
+        enc f32 [B, T, d_model], enc_len i32 [B], targets i32 [B, U_max] (ids in [0, vocab_size)), tgt_len i32 [B] ->
+        (frames i32 [B, U_max]: encoder frame of every token on the Viterbi path, tok_logp f32 [B, U_max]: its log p,
+        viterbi f64 [B], loglik f64 [B]: the log-likelihood summed over all alignments = -RNN-T loss
+        [, lattice f32 [B, T, U_max + 1, 2]: (log p(blank), log p(next target)) of every node]).  Synchronises."""
+        B, T, _ = enc.shape
+        assert enc.dtype == torch.float32 and enc.is_contiguous() and enc_len.dtype == torch.int32
+        assert targets.dtype == torch.int32 and targets.is_contiguous() and targets.dim() == 2 and tgt_len.dtype == torch.int32
+        U = targets.shape[1]
+        frames = torch.empty(B, U, dtype=torch.int32, device=self.device)
+        tok_logp = torch.empty(B, U, dtype=torch.float32, device=self.device)
+        viterbi = torch.empty(B, dtype=torch.float64, device=self.device)
+        loglik = torch.empty(B, dtype=torch.float64, device=self.device)
+        lat = torch.empty(B, T, U + 1, 2, dtype=torch.float32, device=self.device) if lattice else None
+        self._check(self.lib.rs_rnnt_align(self.h, enc.data_ptr(), enc_len.data_ptr(), B, T, targets.data_ptr(), tgt_len.data_ptr(), U,
+                                           frames.data_ptr(), tok_logp.data_ptr(), viterbi.data_ptr(), loglik.data_ptr(),
+                                           lat.data_ptr() if lattice else None, self._stream()), "rs_rnnt_align")
+        return (frames, tok_logp, viterbi, loglik, lat) if lattice else (frames, tok_logp, viterbi, loglik)
 
     def resample_mono(self, raw: torch.Tensor, lens: torch.Tensor, samplerate: int, pad: int = 0):
         """norm_audio on the device (pkg/nemo-asr/src/audio.py:54-68) + transcribe()'s padding: ``raw`` [B, C, L] float32 or

@@ -9,6 +9,9 @@ Same contract as the reference's ``reazonspeech-nemo-asr`` entry point (pkg/nemo
                        (see writer.get_writer)
   no AUDIO argument    "no audio file specified" + usage on stderr, exit status 1
   unknown option       getopt.GetoptError propagates, as in the reference
+  --align=FILE         forced alignment instead of recognition: FILE holds one transcript line per AUDIO argument, in
+                       order; the segments are timed by where the audio says that text.  A line count that differs from
+                       the number of AUDIO arguments prints a message on stderr, exit status 1
 
 One extension: several AUDIO arguments are transcribed as one batch on the GPU (the reference reads exactly one);
 their segments are written one file after the other through the same writer, every file's times shifted by the total
@@ -23,7 +26,7 @@ from dataclasses import dataclass, field
 from typing import List, Optional
 
 SHORT_OPTS = "ho:"
-LONG_OPTS = ("help", "output=", "to=")
+LONG_OPTS = ("help", "output=", "to=", "align=")
 
 
 @dataclass
@@ -32,6 +35,7 @@ class Options:
     output: Optional[str] = None
     fmt: Optional[str] = None
     audio: List[str] = field(default_factory=list)
+    align: Optional[str] = None
 
 
 def parse(argv) -> Options:
@@ -45,6 +49,8 @@ def parse(argv) -> Options:
             opt.output = value
         if flag == "--to":
             opt.fmt = value
+        if flag == "--align":
+            opt.align = value
     return opt
 
 
@@ -52,16 +58,24 @@ def usage() -> None:
     print(__doc__, file=sys.stderr)
 
 
-def run(opt: Options) -> None:
+def read_transcripts(path: str) -> List[str]:
+    with open(path, encoding="utf-8") as f:
+        return [line.rstrip("\r\n") for line in f]
+
+
+def run(opt: Options, transcripts: Optional[List[str]] = None) -> None:
     from .audio import audio_from_path
-    from .transcribe import load_model, transcribe, transcribe_batch
+    from .transcribe import align_batch, load_model, transcribe, transcribe_batch
     from .writer import get_writer
 
     sink = sys.stdout if opt.output is None else open(opt.output, "w")
     warnings.simplefilter("ignore")
     clips = [audio_from_path(path) for path in opt.audio]
-    model = load_model()
-    results = transcribe_batch(model, clips) if len(clips) > 1 else [transcribe(model, clips[0])]
+    if transcripts is not None:
+        results = align_batch(load_model(aligner=True), clips, transcripts)
+    else:
+        model = load_model()
+        results = transcribe_batch(model, clips) if len(clips) > 1 else [transcribe(model, clips[0])]
     with sink:
         out = get_writer(sink, opt.fmt)
         out.write_header()
@@ -82,7 +96,14 @@ def main(argv=None):
         print("no audio file specified", file=sys.stderr)
         usage()
         return 1
-    run(opt)
+    transcripts = None
+    if opt.align is not None:
+        transcripts = read_transcripts(opt.align)
+        if len(transcripts) != len(opt.audio):
+            print(f"{opt.align}: {len(transcripts)} transcript lines for {len(opt.audio)} audio files (--align wants one line per file)",
+                  file=sys.stderr)
+            return 1
+    run(opt, transcripts)
     return None
 
 

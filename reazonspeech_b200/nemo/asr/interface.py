@@ -67,6 +67,17 @@ class TranscribeResult:
 
 
 @dataclass
+class AlignResult(TranscribeResult):
+    """What ``align`` / ``align_batch`` return: the transcript's subwords and segments timed by the most likely alignment, plus
+    ``log_likelihood`` (log p(text | audio) summed over every alignment: minus the RNN-T loss), ``viterbi_log_prob`` (log p of
+    the best alignment alone) and ``token_log_probs`` (log p of every target token where that alignment emits it; one entry
+    per token id, including ids that decode to no text and so have no subword)."""
+    log_likelihood: float = 0.0
+    viterbi_log_prob: float = 0.0
+    token_log_probs: List[float] = field(default_factory=list)
+
+
+@dataclass
 class TranscribeConfig:
     verbose: bool = True
     raw_hypothesis: bool = False

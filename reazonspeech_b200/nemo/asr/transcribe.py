@@ -12,7 +12,7 @@ from __future__ import annotations
 import glob
 import os
 from dataclasses import dataclass
-from typing import List, Optional, Sequence
+from typing import List, Optional, Sequence, Union
 
 import numpy as np
 import torch
@@ -23,7 +23,7 @@ from ...tokenizer import PieceTableTokenizer, SentencePieceTokenizer, synthetic_
 from ...weights import load_nemo_archive, random_state_dict
 from .audio import SAMPLERATE, norm_audio, pad_audio
 from .decode import PAD_SECONDS, build_result, decode_hypothesis
-from .interface import AudioData, TranscribeConfig, TranscribeResult
+from .interface import AlignResult, AudioData, TranscribeConfig, TranscribeResult
 
 HF_REPO = "reazon-research/reazonspeech-nemo-v2"
 ENV_CHECKPOINT = "REAZONSPEECH_NEMO_CHECKPOINT"
@@ -214,6 +214,38 @@ class B200RnntModel:
                 out[i] = Hypothesis(y[r, : k + 1].to(torch.long), steps[r, :k].tolist(), float(score[r]))
         return out
 
+    def align_tokens(self, waveforms: Sequence[np.ndarray], token_lists: Sequence[Sequence[int]], pad: int = 0):
+        """RNN-T forced alignment of known token sequences (rs_rnnt_align): 16 kHz mono waveforms (each gets ``pad`` zero
+        samples on both sides) and one token-id list per waveform -> ``[(frames, token_log_probs, viterbi_log_prob,
+        log_likelihood)]`` in input order; ``frames[i]`` is the encoder frame that emits token i on the best path.  Batches are
+        cut by length, as in ``transcribe_alsd``."""
+        eng = self.engine
+        if "alsd.out.w3" not in eng.weights:
+            raise RuntimeError("this model was loaded without the aligner weights: load it with load_model(..., aligner=True)")
+        if len(token_lists) != len(waveforms):
+            raise ValueError(f"align_tokens: {len(waveforms)} waveforms but {len(token_lists)} token lists")
+        out: List[Optional[tuple]] = [None] * len(waveforms)
+        order = sorted(range(len(waveforms)), key=lambda i: len(waveforms[i]))
+        for lo in range(0, len(order), self.max_batch):
+            idx = order[lo:lo + self.max_batch]
+            wav, lens = self._staging[0].stage([waveforms[i] for i in idx], pad)
+            U = max(1, max(len(token_lists[i]) for i in idx))
+            targets = torch.zeros(len(idx), U, dtype=torch.int32)
+            for r, i in enumerate(idx):
+                targets[r, : len(token_lists[i])] = torch.tensor([int(t) for t in token_lists[i]], dtype=torch.int32)
+            tgt_len = torch.tensor([len(token_lists[i]) for i in idx], dtype=torch.int32)
+            with torch.cuda.device(eng.device):
+                x = wav.to(eng.device, non_blocking=True)
+                if x.dtype == torch.int16:
+                    x = x.to(torch.float32) * (1.0 / 32768.0)
+                mel, mel_len = eng.log_mel(x, lens.to(eng.device))
+                enc, enc_len = eng.encode(mel, mel_len)
+                frames, tok_logp, viterbi, loglik = [a.cpu() for a in eng.align(enc, enc_len, targets.to(eng.device), tgt_len.to(eng.device))]
+            for r, i in enumerate(idx):
+                k = len(token_lists[i])
+                out[i] = (frames[r, :k].tolist(), tok_logp[r, :k].tolist(), float(viterbi[r]), float(loglik[r]))
+        return out
+
     def transcribe(self, audio, batch_size: int = 1, return_hypotheses: bool = True, verbose: bool = True, **_):
         waves = [a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a) for a in audio]
         if self.decoding == "alsd":
@@ -236,7 +268,7 @@ def _find_checkpoint() -> Optional[str]:
 
 def load_model(device=None, *, checkpoint: Optional[str] = None, synthetic: Optional[bool] = None,
                config: Optional[ModelConfig] = None, seed: int = 0, max_batch: int = 64, devices: Optional[Sequence] = None,
-               decoding: str = "greedy", beam_size: int = 4):
+               decoding: str = "greedy", beam_size: int = 4, aligner: bool = False):
     """Load the ReazonSpeech FastConformer-RNNT onto a B200.
 
     ``device``: None / "cuda" / "cuda:N" as in the reference (transcribe.py:9-22, eval.py:26).
@@ -245,7 +277,8 @@ def load_model(device=None, *, checkpoint: Optional[str] = None, synthetic: Opti
     (pkg/nemo-asr/src/decode.py:29); it runs on the GPU too (csrc/decode_alsd.cu).  ``devices`` (e.g. ``range(8)`` or ``["cuda:0", "cuda:1"]``) loads one
     replica per listed GPU into THIS process and returns a model that deals every call's utterances across them
     (``multi_gpu.MultiGpuRnntModel``; same surface, results in input order).  Weights come from ``checkpoint`` (a .nemo file),
-    $REAZONSPEECH_NEMO_CHECKPOINT or the local Hugging Face cache of reazonspeech-nemo-v2.
+    $REAZONSPEECH_NEMO_CHECKPOINT or the local Hugging Face cache of reazonspeech-nemo-v2.  ``aligner=True`` uploads the
+    weights ``align`` / ``align_batch`` need (the tripled predictor / joint matrices, as ``decoding="alsd"`` does).
     With ``synthetic=True`` (or $REAZONSPEECH_B200_SYNTHETIC=1) seeded random weights of the same
     architecture are used instead -- the only option offline."""
     if device is None:
@@ -273,9 +306,12 @@ def load_model(device=None, *, checkpoint: Optional[str] = None, synthetic: Opti
     if decoding not in ("greedy", "alsd"):
         raise ValueError(f"decoding must be 'greedy' or 'alsd', got {decoding!r}")
     if devices is None:
-        return B200RnntModel(Engine(cfg, sd, str(device), alsd=decoding == "alsd"), tokenizer, max_batch=max_batch, decoding=decoding, beam_size=beam_size)
+        return B200RnntModel(Engine(cfg, sd, str(device), alsd=decoding == "alsd" or aligner), tokenizer, max_batch=max_batch,
+                             decoding=decoding, beam_size=beam_size)
     if decoding != "greedy":
         raise ValueError("the one-process multi-GPU model decodes greedily; load one model per device for beam search")
+    if aligner:
+        raise NotImplementedError("the one-process multi-GPU model does not align; load one model per device for align()")
     names = [d if isinstance(d, str) else f"cuda:{int(d)}" for d in devices]
     if len(names) == 0 or len(set(names)) != len(names):
         raise ValueError(f"devices must name distinct GPUs, got {list(devices)!r}")
@@ -340,4 +376,31 @@ def transcribe_batch(model, audios: Sequence[AudioData], config: Optional[Transc
         hyps = model.transcribe(tensors, batch_size=max(len(tensors), 1), return_hypotheses=True, verbose=config.verbose)
         for i, hyp in enumerate(hyps):
             finish(i, hyp)
+    return out
+
+
+def align(model, audio: AudioData, text: Union[str, Sequence[int]], config: Optional[TranscribeConfig] = None) -> AlignResult:
+    """When is a known transcript said in ``audio``, and how well does the audio support it: RNN-T forced alignment of
+    ``text`` (a string, tokenised with ``model.tokenizer.text_to_ids``, or a list of token ids).  The audio is prepared as
+    ``transcribe`` prepares it (norm_audio, 0.5 s of silence on both sides); subwords and segments carry the times of the
+    frames that emit the tokens on the most likely alignment.  Needs ``load_model(..., aligner=True)``."""
+    return align_batch(model, [audio], [text], config)[0]
+
+
+def align_batch(model, audios: Sequence[AudioData], texts: Sequence[Union[str, Sequence[int]]],
+                config: Optional[TranscribeConfig] = None) -> List[AlignResult]:
+    """``align`` for many utterances through a few engine launches; results in input order."""
+    if config is None:
+        config = TranscribeConfig()
+    if len(texts) != len(audios):
+        raise ValueError(f"align_batch: {len(audios)} audios but {len(texts)} texts")
+    ids = [model.tokenizer.text_to_ids(t) if isinstance(t, str) else [int(i) for i in t] for t in texts]
+    waves = [np.asarray(norm_audio(a).waveform) for a in audios]
+    out: List[AlignResult] = []
+    for tokens, (frames, tok_logp, viterbi, loglik) in zip(ids, model.align_tokens(waves, ids, pad=int(PAD_SECONDS * SAMPLERATE))):
+        steps = [f + i + 1 for i, f in enumerate(frames)]             # Hypothesis.from_greedy's convention
+        r = build_result(model.tokenizer, tokens, steps)
+        out.append(AlignResult(r.text, r.subwords, r.segments,
+                               hypothesis=Hypothesis.from_greedy(tokens, frames, model.cfg.blank) if config.raw_hypothesis else None,
+                               log_likelihood=loglik, viterbi_log_prob=viterbi, token_log_probs=tok_logp))
     return out

@@ -1,5 +1,5 @@
 """Tokenizers exposing NeMo's ``tokenizer.ids_to_text`` (the only tokenizer call the reference
-makes: pkg/nemo-asr/src/decode.py:41,47).
+makes: pkg/nemo-asr/src/decode.py:41,47) and ``text_to_ids`` (what forced alignment tokenises a transcript with).
 
 ``SentencePieceTokenizer`` wraps a real ``tokenizer.model`` from the .nemo archive.
 ``PieceTableTokenizer`` is the stand-in used with synthetic weights: a deterministic table of
@@ -28,6 +28,14 @@ class PieceTableTokenizer:
     def ids_to_pieces(self, ids: Iterable[int]) -> List[str]:
         return [self.pieces[int(i)] for i in ids]
 
+    def text_to_ids(self, text: str) -> List[int]:
+        """One piece per character: a space becomes the word-boundary piece, a character outside the table the unknown
+        piece (id 0).  ``ids_to_text(text_to_ids(s)) == s`` for text of table characters and inner spaces."""
+        index = self.__dict__.get("_index")
+        if index is None:
+            index = self._index = {p: i for i, p in reversed(list(enumerate(self.pieces)))}
+        return [index.get(WORD_BOUNDARY if ch == " " else ch, 0) for ch in text]
+
 
 def synthetic_pieces(vocab_size: int) -> List[str]:
     """Deterministic Japanese-looking piece table: <unk>, the word-boundary mark, punctuation,
@@ -53,3 +61,6 @@ class SentencePieceTokenizer:
 
     def ids_to_text(self, ids: Iterable[int]) -> str:
         return self.sp.decode_ids([int(i) for i in ids])
+
+    def text_to_ids(self, text: str) -> List[int]:
+        return list(self.sp.encode_as_ids(text))
