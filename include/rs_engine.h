@@ -161,6 +161,28 @@ int rs_rnnt_align(rs_engine* e, const float* enc_dev, const int32_t* enc_len_dev
                   int32_t* frames_dev, float* tok_logp_dev, double* viterbi_dev, double* loglik_dev,
                   float* lattice_dev, void* stream);
 
+/* Free-span RNN-T alignment: find each of K known token sequences (captions) inside a frame window of one encoder row, as
+ * when a broadcast caption is searched for in the audio around its display time.  enc f32[B,T_max,d_model] + enc_len i32[B];
+ * span i32[K,3] = (src row, lo, hi): caption k lives somewhere in frames [lo, hi) of row src; targets i32[K,U_max] +
+ * tgt_len i32[K].  The lattice of caption k is rs_rnnt_align's lattice of enc[src, lo:hi] (W = hi - lo frames).  The path may
+ * start at any node (t, 0) at no cost and ends with the closing blank of any frame t_e at u = U:
+ *   alpha(t, 0) = max(0, alpha(t-1, 0) + lb(t-1, 0)),   viterbi = max_t alpha(t, U) + lb(t, U),
+ * and loglik is the same recursion with logaddexp (logsumexp over every (start, end) pair of rs_rnnt_align's loglik), all in
+ * float64.  Ties: at u = 0 an exact tie goes to the fresh start, at the end to the earliest t_e, inside the lattice to the
+ * blank edge (as rs_rnnt_align).  Every log p(blank) <= 0, so the best span is exactly [frames[0], frames[U-1]].
+ * Outputs: frames i32[K,U_max] (ABSOLUTE encoder frame, lo + window frame, of each token on the best path; -1 past tgt_len),
+ * tok_logp f32[K,U_max], path_logp f32[K,F_max] (indexed by window frame t - lo: lb(t, u_t) plus the log p of the tokens the
+ * path emits at t, summed in fp32; 0 outside the span, and the span's entries sum to viterbi up to fp32 rounding),
+ * viterbi f64[K], loglik f64[K], lattice f32[K,F_max,U_max+1,2] (nullable; other entries unspecified).
+ * RS_ERR_INVALID_ARG before any computation when: enc_len[b] outside [0, T_max], src outside [0, B), lo < 0, lo >= hi,
+ * hi > enc_len[src], tgt_len[k] outside [1, U_max], F_max < max(hi - lo), or a target outside [0, vocab_size).
+ * joint.enc runs once over the B * T_max rows and the predictor once over the K captions.  Needs the "alsd.*" weight tensors
+ * (RS_ERR_UNSUPPORTED without them).  Synchronises before returning. */
+int rs_rnnt_align_spans(rs_engine* e, const float* enc_dev, const int32_t* enc_len_dev, int B, int T_max, int K,
+                        const int32_t* span_dev, const int32_t* targets_dev, const int32_t* tgt_len_dev, int U_max,
+                        int32_t* frames_dev, float* tok_logp_dev, float* path_logp_dev, int F_max, double* viterbi_dev,
+                        double* loglik_dev, float* lattice_dev, void* stream);
+
 /* norm_audio on the device (pkg/nemo-asr/src/audio.py:54-68: resample to 16 kHz, then average the channels) fused with
  * transcribe()'s padding (audio.py:70-83): in [B, channels, L_in_max] f32 or int16 PCM at the native rate ->
  * out f32 [B, L_out_row], row b = pad zeros | resampled mono utterance | zeros, len_out[b] = resampled length + 2 pad;

@@ -13,6 +13,10 @@
 //     align_lattice   persistent TMA -> tcgen05.mma -> TMEM kernel: one CTA owns a 128-row block across all N blocks and
 //                     reduces the logits to (log p(blank), log p(target)) in its epilogue; no logit reaches HBM
 //   align_dp        anti-diagonal sweep per utterance: Viterbi (max) and forward (logaddexp) in float64, backtrace
+//
+// rs_rnnt_align_spans runs the same kernels over K frame windows of the encoder rows (semantics:
+// oracle/align_spans_restated.py): the predictor over the K items, align_rows reading joint.enc rows from a per-item row
+// base (src * T_max + lo; b * T_max for whole utterances), align_dp<kSpan = true> letting the path start and end anywhere.
 #include <cuda.h>
 
 #include <cfloat>
@@ -73,8 +77,8 @@ align_pred_kernel(const float* __restrict__ gates, float* __restrict__ c_state, 
 // grid (n_rows), block 128.  (The lattice kernel's TMA zero-fills the rows of its last tile past n_rows.)
 __global__ void __launch_bounds__(128)
 align_rows_kernel(const float* __restrict__ enc_proj, const float* __restrict__ pred_proj, const int64_t* __restrict__ offs,
-                  const int32_t* __restrict__ tgt_len, const int32_t* __restrict__ targets, int B, int T_max, int U1, int U_max,
-                  int Hj, int64_t r0, __nv_bfloat16* __restrict__ planes, int32_t* __restrict__ tcol) {
+                  const int64_t* __restrict__ row_base, const int32_t* __restrict__ tgt_len, const int32_t* __restrict__ targets,
+                  int B, int U1, int U_max, int Hj, int64_t r0, __nv_bfloat16* __restrict__ planes, int32_t* __restrict__ tcol) {
   const int r = blockIdx.x;
   __nv_bfloat16* row = planes + static_cast<size_t>(r) * 3 * Hj;
   const int64_t n = r0 + r;
@@ -87,7 +91,7 @@ align_rows_kernel(const float* __restrict__ enc_proj, const float* __restrict__ 
   const int64_t local = n - offs[b];
   const int t = static_cast<int>(local / (U + 1)), u = static_cast<int>(local % (U + 1));
   if (threadIdx.x == 0) tcol[r] = u < U ? targets[static_cast<size_t>(b) * U_max + u] : -1;
-  const float4* ep = reinterpret_cast<const float4*>(enc_proj + (static_cast<size_t>(b) * T_max + t) * Hj);
+  const float4* ep = reinterpret_cast<const float4*>(enc_proj + static_cast<size_t>(row_base[b] + t) * Hj);
   const float4* pp = reinterpret_cast<const float4*>(pred_proj + (static_cast<size_t>(b) * U1 + u) * Hj);
   for (int j4 = threadIdx.x; j4 < Hj / 4; j4 += blockDim.x) {
     const float4 a = ep[j4], g = pp[j4];
@@ -276,11 +280,20 @@ __device__ __forceinline__ double logaddexp(double a, double b) {
 // grid (B), block 256.  Anti-diagonal d = t + u; two diagonals of (Viterbi, forward) in shared memory indexed by u.
 // Back-pointer per node: 1 = reached by emitting y_u from (t, u - 1), 0 = by a blank from (t - 1, u), which wins exact ties:
 // the backtrace runs from the last node, so preferring the blank edge moves every token to its earliest frame.
+//
+// kSpan (rs_rnnt_align_spans): item b is the frame window [lo, hi) of span[b], T = hi - lo (enc_len holds T, T_max the row
+// pitch F_max of path_logp and lattice).  The path may start at any node (t, 0) at no cost -- back-pointer 2, which wins an
+// exact tie with the blank edge -- and ends with the closing blank of any frame t_e at u = U.  The end terms are folded in
+// ascending t by whichever thread owns the diagonal's node (t, U): a strict running max (the earliest t_e wins a tie) and a
+// running logaddexp, in shared memory after the four diagonals.  The backtrace runs from (t_e, U) to the first start state;
+// frames are reported as lo + t, and path_logp[b, t] of every frame of the span is lb(t, u_t) plus the ly of the tokens the
+// path emits at t, summed in fp32 in that order (the blank, then the tokens from the last to the first); 0 elsewhere.
+template <bool kSpan>
 __global__ void __launch_bounds__(256)
 align_dp_kernel(const float2* __restrict__ lp, const int64_t* __restrict__ offs, const int32_t* __restrict__ enc_len,
                 const int32_t* __restrict__ tgt_len, int T_max, int U_max, int U1, uint8_t* __restrict__ bp_all,
                 int32_t* __restrict__ frames, float* __restrict__ tok_logp, double* __restrict__ viterbi, double* __restrict__ loglik,
-                float* __restrict__ lattice) {
+                float* __restrict__ lattice, const int32_t* __restrict__ span, float* __restrict__ path_logp) {
   extern __shared__ double dp_smem[];
   const int b = blockIdx.x;
   const int T = enc_len[b], U = tgt_len[b], W = U + 1;
@@ -288,6 +301,8 @@ align_dp_kernel(const float2* __restrict__ lp, const int64_t* __restrict__ offs,
   uint8_t* P = bp_all + offs[b];
   auto av = [&](int i) { return dp_smem + i * U1; };             // [Viterbi even | Viterbi odd | forward even | forward odd]
   auto af = [&](int i) { return dp_smem + (2 + i) * U1; };
+  double* end_acc = dp_smem + 4 * U1;                            // kSpan: [Viterbi end max, forward end sum], then t_e
+  int* end_t = reinterpret_cast<int*>(end_acc + 2);
   if (lattice != nullptr) {
     for (int i = threadIdx.x; i < T * W; i += blockDim.x) {
       const int t = i / W, u = i % W;
@@ -299,6 +314,9 @@ align_dp_kernel(const float2* __restrict__ lp, const int64_t* __restrict__ offs,
   for (int u = U + threadIdx.x; u < U_max; u += blockDim.x) {
     frames[static_cast<size_t>(b) * U_max + u] = -1;
     tok_logp[static_cast<size_t>(b) * U_max + u] = 0.f;
+  }
+  if constexpr (kSpan) {
+    for (int t = threadIdx.x; t < T_max; t += blockDim.x) path_logp[static_cast<size_t>(b) * T_max + t] = 0.f;
   }
   for (int d = 0; d < T + U; ++d) {
     const double* pv = av((d & 1) ^ 1); const double* pf = af((d & 1) ^ 1);
@@ -320,25 +338,67 @@ align_dp_kernel(const float2* __restrict__ lp, const int64_t* __restrict__ offs,
       } else if (t > 0) {
         const double lb = static_cast<double>(L[(t - 1) * W + u].x);
         v = pv[u] + lb; f = pf[u] + lb;
+        if constexpr (kSpan) {                                   // fresh start at (t, 0): 0, wins an exact tie
+          e = v > 0.0 ? 0 : 2;
+          v = e ? 0.0 : v;
+          f = logaddexp(0.0, f);
+        }
+      } else if constexpr (kSpan) {
+        e = 2;
       }
       cv[u] = v; cf[u] = f;
       P[t * W + u] = e;
+      if constexpr (kSpan) {
+        if (u == U) {                                            // one node per diagonal, diagonals in ascending t
+          const double lb_end = static_cast<double>(L[t * W + U].x);
+          const double ve = v + lb_end, fe = f + lb_end;
+          if (t == 0) {
+            end_acc[0] = ve; end_acc[1] = fe; *end_t = 0;
+          } else {
+            if (ve > end_acc[0]) { end_acc[0] = ve; *end_t = t; }
+            end_acc[1] = logaddexp(end_acc[1], fe);
+          }
+        }
+      }
     }
     __syncthreads();
   }
   if (threadIdx.x != 0) return;
-  const int dl = T - 1 + U;
-  const double lb_end = static_cast<double>(L[(T - 1) * W + U].x);
-  viterbi[b] = av(dl & 1)[U] + lb_end;
-  loglik[b] = af(dl & 1)[U] + lb_end;
-  int t = T - 1, u = U;
-  while (u > 0) {
-    if (P[t * W + u]) {
-      --u;
-      frames[static_cast<size_t>(b) * U_max + u] = t;
-      tok_logp[static_cast<size_t>(b) * U_max + u] = L[t * W + u].y;
-    } else {
-      --t;
+  if constexpr (kSpan) {
+    viterbi[b] = end_acc[0];
+    loglik[b] = end_acc[1];
+    const int lo = span[3 * b + 1];
+    int t = *end_t, u = U;
+    float acc = L[t * W + U].x;
+    for (;;) {
+      const uint8_t p = P[t * W + u];
+      if (p == 1) {
+        --u;
+        const float y = L[t * W + u].y;
+        frames[static_cast<size_t>(b) * U_max + u] = lo + t;
+        tok_logp[static_cast<size_t>(b) * U_max + u] = y;
+        acc += y;
+      } else {
+        path_logp[static_cast<size_t>(b) * T_max + t] = acc;
+        if (p == 2) break;
+        --t;
+        acc = L[t * W + u].x;
+      }
+    }
+  } else {
+    const int dl = T - 1 + U;
+    const double lb_end = static_cast<double>(L[(T - 1) * W + U].x);
+    viterbi[b] = av(dl & 1)[U] + lb_end;
+    loglik[b] = af(dl & 1)[U] + lb_end;
+    int t = T - 1, u = U;
+    while (u > 0) {
+      if (P[t * W + u]) {
+        --u;
+        frames[static_cast<size_t>(b) * U_max + u] = t;
+        tok_logp[static_cast<size_t>(b) * U_max + u] = L[t * W + u].y;
+      } else {
+        --t;
+      }
     }
   }
 }
@@ -360,9 +420,10 @@ cudaError_t align_pred(const float* gates, float* c_state, const int32_t* target
   return cudaGetLastError();
 }
 
-cudaError_t align_rows(const float* enc_proj, const float* pred_proj, const int64_t* offs, const int32_t* tgt_len, const int32_t* targets,
-                       int B, int T_max, int U1, int U_max, int Hj, int64_t r0, int n_rows, void* planes, int32_t* tcol, cudaStream_t s) {
-  align_rows_kernel<<<n_rows, 128, 0, s>>>(enc_proj, pred_proj, offs, tgt_len, targets, B, T_max, U1, U_max, Hj, r0,
+cudaError_t align_rows(const float* enc_proj, const float* pred_proj, const int64_t* offs, const int64_t* row_base,
+                       const int32_t* tgt_len, const int32_t* targets, int B, int U1, int U_max, int Hj, int64_t r0, int n_rows,
+                       void* planes, int32_t* tcol, cudaStream_t s) {
+  align_rows_kernel<<<n_rows, 128, 0, s>>>(enc_proj, pred_proj, offs, row_base, tgt_len, targets, B, U1, U_max, Hj, r0,
                                            static_cast<__nv_bfloat16*>(planes), tcol);
   return cudaGetLastError();
 }
@@ -389,22 +450,36 @@ cudaError_t align_lattice(const void* planes, const void* w3, const float* bias,
   return cudaGetLastError();
 }
 
-size_t align_dp_smem_bytes(int U1) { return static_cast<size_t>(4) * U1 * sizeof(double); }
+size_t align_dp_smem_bytes(int U1, bool span) { return static_cast<size_t>(4) * U1 * sizeof(double) + (span ? 32 : 0); }
 
-cudaError_t align_dp(const float2* lp, const int64_t* offs, const int32_t* enc_len, const int32_t* tgt_len, int B, int T_max,
-                     int U_max, int U1, uint8_t* bp, int32_t* frames, float* tok_logp, double* viterbi, double* loglik, float* lattice,
-                     cudaStream_t s) {
-  const size_t smem = align_dp_smem_bytes(U1);
+namespace {
+template <bool kSpan>
+cudaError_t launch_dp(const float2* lp, const int64_t* offs, const int32_t* enc_len, const int32_t* tgt_len, int B, int T_max,
+                      int U_max, int U1, uint8_t* bp, int32_t* frames, float* tok_logp, double* viterbi, double* loglik, float* lattice,
+                      const int32_t* span, float* path_logp, cudaStream_t s) {
+  const size_t smem = align_dp_smem_bytes(U1, kSpan);
   if (smem > 48 * 1024) {
     static DeviceOnce attr_once;
     if (attr_once.pending()) {
-      cudaError_t e = cudaFuncSetAttribute(align_dp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+      cudaError_t e = cudaFuncSetAttribute(align_dp_kernel<kSpan>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
       if (e != cudaSuccess) return e;
       attr_once.set();
     }
   }
-  align_dp_kernel<<<B, 256, smem, s>>>(lp, offs, enc_len, tgt_len, T_max, U_max, U1, bp, frames, tok_logp, viterbi, loglik, lattice);
+  align_dp_kernel<kSpan><<<B, 256, smem, s>>>(lp, offs, enc_len, tgt_len, T_max, U_max, U1, bp, frames, tok_logp, viterbi, loglik,
+                                              lattice, span, path_logp);
   return cudaGetLastError();
+}
+}  // namespace
+
+cudaError_t align_dp(const float2* lp, const int64_t* offs, const int32_t* enc_len, const int32_t* tgt_len, int B, int T_max,
+                     int U_max, int U1, uint8_t* bp, int32_t* frames, float* tok_logp, double* viterbi, double* loglik, float* lattice,
+                     const int32_t* span, float* path_logp, cudaStream_t s) {
+  return span != nullptr
+             ? launch_dp<true>(lp, offs, enc_len, tgt_len, B, T_max, U_max, U1, bp, frames, tok_logp, viterbi, loglik, lattice, span,
+                               path_logp, s)
+             : launch_dp<false>(lp, offs, enc_len, tgt_len, B, T_max, U_max, U1, bp, frames, tok_logp, viterbi, loglik, lattice,
+                                nullptr, nullptr, s);
 }
 
 }  // namespace rs

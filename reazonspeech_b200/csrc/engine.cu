@@ -715,44 +715,43 @@ int rs_rnnt_alsd(rs_engine* e, const float* enc, const int32_t* enc_len, int B, 
   return RS_OK;
 }
 
-// RNN-T forced alignment of given token sequences (align.cu; semantics: oracle/align_restated.py).  The lengths are read back
-// once to lay out the compact node list (utterance b: T_b * (U_b + 1) nodes); the lattice is evaluated in chunks of
-// kAlignChunkRows nodes so that the bf16 A planes stay bounded.  Synchronises.
-int rs_rnnt_align(rs_engine* e, const float* enc, const int32_t* enc_len, int B, int T_max, const int32_t* targets,
-                  const int32_t* tgt_len, int U_max, int32_t* frames, float* tok_logp, double* viterbi, double* loglik, float* lattice,
-                  void* stream) {
-  if (!e || !enc || !enc_len || !targets || !tgt_len || !frames || !tok_logp || !viterbi || !loglik || B <= 0 || T_max <= 0 || U_max <= 0)
-    return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: bad arguments");
-  if (B > rs_engine::kMaxBatch) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: batch of %d utterances exceeds the engine limit of %d", B, rs_engine::kMaxBatch);
-  if (e->alsd.out_w3 == nullptr)
-    return fail(e, RS_ERR_UNSUPPORTED, "rs_rnnt_align: the engine was created without the aligner weight tensors (alsd.*)");
-  RS_CUDA(e, cudaSetDevice(e->device));
-  Nvtx range("rs::rnnt_align");
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
+namespace {
+
+// The items of one forced-alignment pass, laid out on the host after the argument checks: item i aligns targets[i, :U[i]]
+// against T[i] rows of the joint.enc projection starting at row row_base[i].
+struct AlignItems {
+  std::vector<int32_t> T, U;
+  std::vector<int64_t> row_base;
+  const int32_t* T_dev = nullptr;      // T on the device (enc_len of whole utterances); nullptr: uploaded from T
+  const int32_t* span = nullptr;       // [n, 3] (src, lo, hi) on the device: free-span DP; nullptr: whole utterances
+};
+
+// Node layout, workspace, joint.enc over the M encoder rows, teacher-forced predictor over the items, chunked lattice and DP
+// (align.cu).  The lattice is evaluated in chunks of kAlignChunkRows nodes so that the bf16 A planes stay bounded.  T_pitch is
+// the row pitch of lattice and path_logp.  Synchronises.
+int align_run(rs_engine* e, const char* fn, const float* enc, int M, const AlignItems& it, const int32_t* targets,
+              const int32_t* tgt_len, int U_max, int T_pitch, int32_t* frames, float* tok_logp, float* path_logp, double* viterbi,
+              double* loglik, float* lattice, cudaStream_t s) {
   const rs_model_config& c = e->cfg;
   const int Hj = c.joint_hidden, Hp = c.pred_hidden, d = c.d_model, V = c.vocab_size, n_pad = e->alsd.n_pad;
-  std::vector<int32_t> T(B), U(B);
-  RS_CUDA(e, cudaMemcpyAsync(T.data(), enc_len, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, s));
-  RS_CUDA(e, cudaMemcpyAsync(U.data(), tgt_len, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, s));
-  RS_CUDA(e, cudaStreamSynchronize(s));
+  const int B = static_cast<int>(it.T.size());
   std::vector<int64_t> offs(B + 1, 0);
   int U_top = 0;
   for (int b = 0; b < B; ++b) {
-    if (T[b] < 1 || T[b] > T_max) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: enc_len[%d] = %d outside [1, T_max = %d]", b, T[b], T_max);
-    if (U[b] < 0 || U[b] > U_max) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: tgt_len[%d] = %d outside [0, U_max = %d]", b, U[b], U_max);
-    offs[b + 1] = offs[b] + static_cast<int64_t>(T[b]) * (U[b] + 1);
-    U_top = std::max(U_top, U[b]);
+    offs[b + 1] = offs[b] + static_cast<int64_t>(it.T[b]) * (it.U[b] + 1);
+    U_top = std::max(U_top, it.U[b]);
   }
-  const int U1 = U_top + 1;                                // predictor states h_0 .. h_U per utterance
-  if (rs::align_dp_smem_bytes(U1) > 227 * 1024)
-    return fail(e, RS_ERR_UNSUPPORTED, "rs_rnnt_align: %d targets in one utterance exceed what the DP kernel holds in shared memory (%d)",
-                U_top, static_cast<int>(227 * 1024 / rs::align_dp_smem_bytes(1)) - 1);
+  const int U1 = U_top + 1;                                // predictor states h_0 .. h_U per item
+  const bool span = it.span != nullptr;
+  if (rs::align_dp_smem_bytes(U1, span) > 227 * 1024)
+    return fail(e, RS_ERR_UNSUPPORTED, "%s: %d targets in one utterance exceed what the DP kernel holds in shared memory (%d)", fn,
+                U_top, static_cast<int>((227 * 1024 - rs::align_dp_smem_bytes(0, span)) / rs::align_dp_smem_bytes(1)) - 1);
   const int64_t total = offs[B];
   const int chunk = static_cast<int>(std::min<int64_t>(total, rs::kAlignChunkRows));
-  const int M = B * T_max;
   // ---- workspace
   Arena a;
-  const size_t o_flag = a.take(256), o_offs = a.take(static_cast<size_t>(B + 1) * 8);
+  const size_t o_flag = a.take(256), o_offs = a.take(static_cast<size_t>(B + 1) * 8), o_base = a.take(static_cast<size_t>(B) * 8);
+  const size_t o_T = a.take(it.T_dev ? 0 : static_cast<size_t>(B) * 4);
   const size_t o_xn = a.take(static_cast<size_t>(M) * d * 2), o_encp = a.take(static_cast<size_t>(M) * Hj * 4);
   const size_t o_in = a.take(static_cast<size_t>(B) * 6 * Hp * 2), o_gates = a.take(static_cast<size_t>(B) * 4 * Hp * 4);
   const size_t o_c = a.take(static_cast<size_t>(B) * Hp * 4), o_hp = a.take(static_cast<size_t>(B) * U1 * 3 * Hp * 2);
@@ -768,6 +767,8 @@ int rs_rnnt_align(rs_engine* e, const float* enc, const int32_t* enc_len, int B,
   char* ws = static_cast<char*>(e->align_ws);
   int* flag = reinterpret_cast<int*>(ws + o_flag);
   const int64_t* offs_dev = reinterpret_cast<const int64_t*>(ws + o_offs);
+  const int64_t* base_dev = reinterpret_cast<const int64_t*>(ws + o_base);
+  const int32_t* T_dev = it.T_dev ? it.T_dev : reinterpret_cast<const int32_t*>(ws + o_T);
   float* encp = reinterpret_cast<float*>(ws + o_encp); float* gates = reinterpret_cast<float*>(ws + o_gates);
   float* g = reinterpret_cast<float*>(ws + o_g); float2* lp = reinterpret_cast<float2*>(ws + o_lp);
   // ---- targets outside [0, V) are reported before any kernel indexes a table with them
@@ -776,9 +777,11 @@ int rs_rnnt_align(rs_engine* e, const float* enc, const int32_t* enc_len, int B,
   int bad = 0;
   RS_CUDA(e, cudaMemcpyAsync(&bad, flag, 4, cudaMemcpyDeviceToHost, s));
   RS_CUDA(e, cudaStreamSynchronize(s));
-  if (bad) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: a target id lies outside [0, vocab_size = %d)", V);
+  if (bad) return fail(e, RS_ERR_INVALID_ARG, "%s: a target id lies outside [0, vocab_size = %d)", fn, V);
   RS_CUDA(e, cudaMemcpyAsync(ws + o_offs, offs.data(), static_cast<size_t>(B + 1) * 8, cudaMemcpyHostToDevice, s));
-  // ---- joint.enc over every frame (as in the greedy path)
+  RS_CUDA(e, cudaMemcpyAsync(ws + o_base, it.row_base.data(), static_cast<size_t>(B) * 8, cudaMemcpyHostToDevice, s));
+  if (!it.T_dev) RS_CUDA(e, cudaMemcpyAsync(ws + o_T, it.T.data(), static_cast<size_t>(B) * 4, cudaMemcpyHostToDevice, s));
+  // ---- joint.enc over every encoder row (as in the greedy path)
   RS_K(e, s, rs::launch_f32_to_bf16(enc, ws + o_xn, static_cast<int64_t>(M) * d, s), 1);
   RS_TRY(gemm(e, ws + o_xn, e->dec.enc_w, e->dec.enc_b, nullptr, encp, M, Hj, d, RS_EPI_BIAS_F32, 1.f, s));
   // ---- teacher-forced predictor: step 0 consumes the blank (zero input, zero state), step k the target y_k
@@ -792,17 +795,90 @@ int rs_rnnt_align(rs_engine* e, const float* enc, const int32_t* enc_len, int B,
   // ---- lattice, chunk by chunk
   for (int64_t r0 = 0; r0 < total; r0 += chunk) {
     const int n = static_cast<int>(std::min<int64_t>(chunk, total - r0));
-    RS_K(e, s, rs::align_rows(encp, g, offs_dev, tgt_len, targets, B, T_max, U1, U_max, Hj, r0, n, ws + o_planes,
+    RS_K(e, s, rs::align_rows(encp, g, offs_dev, base_dev, tgt_len, targets, B, U1, U_max, Hj, r0, n, ws + o_planes,
                               reinterpret_cast<int32_t*>(ws + o_tcol), s), 1);
     RS_TRY(launch(e, s, "rs::align_lattice", 1, 0.0, [&](char* msg) {
       return rs::align_lattice(ws + o_planes, e->alsd.out_w3, e->alsd.out_b, reinterpret_cast<const int32_t*>(ws + o_tcol), lp + r0, n,
                                n_pad, Hj, V, e->num_sms, s, msg);
     }));
   }
-  RS_K(e, s, rs::align_dp(lp, offs_dev, enc_len, tgt_len, B, T_max, U_max, U1, reinterpret_cast<uint8_t*>(ws + o_bp), frames, tok_logp,
-                          viterbi, loglik, lattice, s), 1);
+  RS_K(e, s, rs::align_dp(lp, offs_dev, T_dev, tgt_len, B, T_pitch, U_max, U1, reinterpret_cast<uint8_t*>(ws + o_bp), frames, tok_logp,
+                          viterbi, loglik, lattice, it.span, path_logp, s), 1);
   RS_CUDA(e, cudaStreamSynchronize(s));
   return RS_OK;
+}
+
+}  // namespace
+
+// RNN-T forced alignment of given token sequences (align.cu; semantics: oracle/align_restated.py).  The lengths are read back
+// once to lay out the compact node list (utterance b: T_b * (U_b + 1) nodes).  Synchronises.
+int rs_rnnt_align(rs_engine* e, const float* enc, const int32_t* enc_len, int B, int T_max, const int32_t* targets,
+                  const int32_t* tgt_len, int U_max, int32_t* frames, float* tok_logp, double* viterbi, double* loglik, float* lattice,
+                  void* stream) {
+  if (!e || !enc || !enc_len || !targets || !tgt_len || !frames || !tok_logp || !viterbi || !loglik || B <= 0 || T_max <= 0 || U_max <= 0)
+    return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: bad arguments");
+  if (B > rs_engine::kMaxBatch) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: batch of %d utterances exceeds the engine limit of %d", B, rs_engine::kMaxBatch);
+  if (e->alsd.out_w3 == nullptr)
+    return fail(e, RS_ERR_UNSUPPORTED, "rs_rnnt_align: the engine was created without the aligner weight tensors (alsd.*)");
+  RS_CUDA(e, cudaSetDevice(e->device));
+  Nvtx range("rs::rnnt_align");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  AlignItems it;
+  it.T.resize(B); it.U.resize(B); it.row_base.resize(B);
+  RS_CUDA(e, cudaMemcpyAsync(it.T.data(), enc_len, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, s));
+  RS_CUDA(e, cudaMemcpyAsync(it.U.data(), tgt_len, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, s));
+  RS_CUDA(e, cudaStreamSynchronize(s));
+  for (int b = 0; b < B; ++b) {
+    if (it.T[b] < 1 || it.T[b] > T_max) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: enc_len[%d] = %d outside [1, T_max = %d]", b, it.T[b], T_max);
+    if (it.U[b] < 0 || it.U[b] > U_max) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align: tgt_len[%d] = %d outside [0, U_max = %d]", b, it.U[b], U_max);
+    it.row_base[b] = static_cast<int64_t>(b) * T_max;
+  }
+  it.T_dev = enc_len;
+  return align_run(e, "rs_rnnt_align", enc, B * T_max, it, targets, tgt_len, U_max, T_max, frames, tok_logp, nullptr, viterbi, loglik,
+                   lattice, s);
+}
+
+// Free-span alignment of K captions inside frame windows of B encoder rows (align.cu; semantics:
+// oracle/align_spans_restated.py).  The spans and lengths are read back once; joint.enc runs once over the B * T_max rows, the
+// predictor once over the K items.  Synchronises.
+int rs_rnnt_align_spans(rs_engine* e, const float* enc, const int32_t* enc_len, int B, int T_max, int K, const int32_t* span,
+                        const int32_t* targets, const int32_t* tgt_len, int U_max, int32_t* frames, float* tok_logp, float* path_logp,
+                        int F_max, double* viterbi, double* loglik, float* lattice, void* stream) {
+  if (!e || !enc || !enc_len || !span || !targets || !tgt_len || !frames || !tok_logp || !path_logp || !viterbi || !loglik || B <= 0 ||
+      T_max <= 0 || K <= 0 || U_max <= 0 || F_max <= 0)
+    return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align_spans: bad arguments");
+  if (B > rs_engine::kMaxBatch || K > rs_engine::kMaxBatch)
+    return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align_spans: %d rows / %d spans exceed the engine limit of %d", B, K, rs_engine::kMaxBatch);
+  if (e->alsd.out_w3 == nullptr)
+    return fail(e, RS_ERR_UNSUPPORTED, "rs_rnnt_align_spans: the engine was created without the aligner weight tensors (alsd.*)");
+  RS_CUDA(e, cudaSetDevice(e->device));
+  Nvtx range("rs::rnnt_align_spans");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  std::vector<int32_t> len(B), sp(static_cast<size_t>(K) * 3);
+  AlignItems it;
+  it.T.resize(K); it.U.resize(K); it.row_base.resize(K);
+  RS_CUDA(e, cudaMemcpyAsync(len.data(), enc_len, static_cast<size_t>(B) * 4, cudaMemcpyDeviceToHost, s));
+  RS_CUDA(e, cudaMemcpyAsync(sp.data(), span, static_cast<size_t>(K) * 12, cudaMemcpyDeviceToHost, s));
+  RS_CUDA(e, cudaMemcpyAsync(it.U.data(), tgt_len, static_cast<size_t>(K) * 4, cudaMemcpyDeviceToHost, s));
+  RS_CUDA(e, cudaStreamSynchronize(s));
+  for (int b = 0; b < B; ++b)
+    if (len[b] < 0 || len[b] > T_max)
+      return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align_spans: enc_len[%d] = %d outside [0, T_max = %d]", b, len[b], T_max);
+  for (int k = 0; k < K; ++k) {
+    const int src = sp[3 * k], lo = sp[3 * k + 1], hi = sp[3 * k + 2];
+    if (src < 0 || src >= B) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align_spans: span[%d] src = %d outside [0, B = %d)", k, src, B);
+    if (lo < 0 || lo >= hi || hi > len[src])
+      return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align_spans: span[%d] window [%d, %d) is empty or outside [0, enc_len[%d] = %d)", k, lo,
+                  hi, src, len[src]);
+    if (hi - lo > F_max) return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align_spans: span[%d] has %d frames > F_max = %d", k, hi - lo, F_max);
+    if (it.U[k] < 1 || it.U[k] > U_max)
+      return fail(e, RS_ERR_INVALID_ARG, "rs_rnnt_align_spans: tgt_len[%d] = %d outside [1, U_max = %d]", k, it.U[k], U_max);
+    it.T[k] = hi - lo;
+    it.row_base[k] = static_cast<int64_t>(src) * T_max + lo;
+  }
+  it.span = span;
+  return align_run(e, "rs_rnnt_align_spans", enc, B * T_max, it, targets, tgt_len, U_max, F_max, frames, tok_logp, path_logp, viterbi,
+                   loglik, lattice, s);
 }
 
 int rs_resample_mono(rs_engine* e, const void* in_dev, int in_is_pcm16, const int32_t* len_in_dev, int B, int channels, int L_in_max,

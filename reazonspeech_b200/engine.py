@@ -68,6 +68,7 @@ SIGNATURES = {
     "rs_resample_mono": (_ip, [_vp, _vp, _ip, _vp, _ip, _ip, _ip, _vp, _ip, _ip, _ip, _ip, _ip, _vp, _ip, _vp, _vp]),
     "rs_rnnt_alsd": (_ip, [_vp, _vp, _vp, _ip, _ip, _ip, _f32, _ip, _ip, _vp, _vp, _vp, _vp, _ip, _vp]),
     "rs_rnnt_align": (_ip, [_vp, _vp, _vp, _ip, _ip, _vp, _vp, _ip, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "rs_rnnt_align_spans": (_ip, [_vp, _vp, _vp, _ip, _ip, _ip, _vp, _vp, _vp, _ip, _vp, _vp, _vp, _ip, _vp, _vp, _vp, _vp]),
     "rs_gemm_bf16": (_ip, [_vp, _vp, _vp, _vp, _vp, _vp, _ip, _ip, _ip, _ip, _f32, _vp]),
     "rs_layernorm": (_ip, [_vp, _vp, _vp, _vp, _vp, _vp, _ip, _ip, _vp]),
     "rs_launch_count": (_i64, [_vp]),
@@ -400,6 +401,34 @@ class Engine:
                                            frames.data_ptr(), tok_logp.data_ptr(), viterbi.data_ptr(), loglik.data_ptr(),
                                            lat.data_ptr() if lattice else None, self._stream()), "rs_rnnt_align")
         return (frames, tok_logp, viterbi, loglik, lat) if lattice else (frames, tok_logp, viterbi, loglik)
+
+    def align_spans(self, enc: torch.Tensor, enc_len: torch.Tensor, spans: torch.Tensor, targets: torch.Tensor, tgt_len: torch.Tensor,
+                    lattice: bool = False):
+        """Free-span RNN-T alignment (rs_rnnt_align_spans): find each of K token sequences somewhere inside a frame window of
+        one encoder row (needs ``Engine(..., alsd=True)``).  enc f32 [B, T, d_model], enc_len i32 [B], spans i32 [K, 3]
+        (src row, lo, hi), targets i32 [K, U_max] (ids in [0, vocab_size)), tgt_len i32 [K] (>= 1) -> (frames i32 [K, U_max]:
+        absolute encoder frame of every token on the best path, tok_logp f32 [K, U_max], path_logp f32 [K, F_max]: per window
+        frame t - lo, the path's log p at that frame (0 outside the span), viterbi f64 [K], loglik f64 [K]
+        [, lattice f32 [K, F_max, U_max + 1, 2]]), F_max = max(hi - lo).  Synchronises."""
+        B, T, _ = enc.shape
+        assert enc.dtype == torch.float32 and enc.is_contiguous() and enc_len.dtype == torch.int32
+        assert targets.dtype == torch.int32 and targets.is_contiguous() and targets.dim() == 2 and tgt_len.dtype == torch.int32
+        assert spans.dtype == torch.int32 and spans.dim() == 2 and spans.shape[1] == 3 and spans.shape[0] == targets.shape[0]
+        K, U = targets.shape
+        F = max(1, int((spans[:, 2] - spans[:, 1]).max())) if K else 1
+        spans = spans.to(self.device).contiguous()
+        frames = torch.empty(K, U, dtype=torch.int32, device=self.device)
+        tok_logp = torch.empty(K, U, dtype=torch.float32, device=self.device)
+        path_logp = torch.empty(K, F, dtype=torch.float32, device=self.device)
+        viterbi = torch.empty(K, dtype=torch.float64, device=self.device)
+        loglik = torch.empty(K, dtype=torch.float64, device=self.device)
+        lat = torch.empty(K, F, U + 1, 2, dtype=torch.float32, device=self.device) if lattice else None
+        self._check(self.lib.rs_rnnt_align_spans(self.h, enc.data_ptr(), enc_len.data_ptr(), B, T, K, spans.data_ptr(), targets.data_ptr(),
+                                                 tgt_len.data_ptr(), U, frames.data_ptr(), tok_logp.data_ptr(), path_logp.data_ptr(), F,
+                                                 viterbi.data_ptr(), loglik.data_ptr(), lat.data_ptr() if lattice else None,
+                                                 self._stream()), "rs_rnnt_align_spans")
+        out = (frames, tok_logp, path_logp, viterbi, loglik)
+        return out + (lat,) if lattice else out
 
     def resample_mono(self, raw: torch.Tensor, lens: torch.Tensor, samplerate: int, pad: int = 0):
         """norm_audio on the device (pkg/nemo-asr/src/audio.py:54-68) + transcribe()'s padding: ``raw`` [B, C, L] float32 or

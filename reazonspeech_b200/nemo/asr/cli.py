@@ -12,6 +12,12 @@ Same contract as the reference's ``reazonspeech-nemo-asr`` entry point (pkg/nemo
   --align=FILE         forced alignment instead of recognition: FILE holds one transcript line per AUDIO argument, in
                        order; the segments are timed by where the audio says that text.  A line count that differs from
                        the number of AUDIO arguments prints a message on stderr, exit status 1
+  --align-captions=FILE
+                       re-time the captions of an SRT or WebVTT FILE against exactly one AUDIO argument: each caption is
+                       searched for from 25 s before its start time to its end time (live captions lag the speech) and
+                       written as one segment with the times where the audio says it.  Captions that cannot be placed are
+                       skipped and counted on stderr.  More or fewer than one AUDIO argument, or --align as well, prints
+                       a message on stderr, exit status 1
 
 One extension: several AUDIO arguments are transcribed as one batch on the GPU (the reference reads exactly one);
 their segments are written one file after the other through the same writer, every file's times shifted by the total
@@ -26,7 +32,7 @@ from dataclasses import dataclass, field
 from typing import List, Optional
 
 SHORT_OPTS = "ho:"
-LONG_OPTS = ("help", "output=", "to=", "align=")
+LONG_OPTS = ("help", "output=", "to=", "align=", "align-captions=")
 
 
 @dataclass
@@ -36,6 +42,7 @@ class Options:
     fmt: Optional[str] = None
     audio: List[str] = field(default_factory=list)
     align: Optional[str] = None
+    align_captions: Optional[str] = None
 
 
 def parse(argv) -> Options:
@@ -51,6 +58,8 @@ def parse(argv) -> Options:
             opt.fmt = value
         if flag == "--align":
             opt.align = value
+        if flag == "--align-captions":
+            opt.align_captions = value
     return opt
 
 
@@ -87,6 +96,28 @@ def run(opt: Options, transcripts: Optional[List[str]] = None) -> None:
             offset += clip.seconds
 
 
+def run_captions(opt: Options) -> None:
+    from .audio import audio_from_path
+    from .captions import read_captions
+    from .interface import Segment
+    from .transcribe import align_captions, load_model
+    from .writer import get_writer
+
+    captions = read_captions(opt.align_captions)
+    sink = sys.stdout if opt.output is None else open(opt.output, "w")
+    warnings.simplefilter("ignore")
+    placed = align_captions(load_model(aligner=True), audio_from_path(opt.audio[0]), captions)
+    with sink:
+        out = get_writer(sink, opt.fmt)
+        out.write_header()
+        for r in placed:
+            if r is not None:
+                out.write(Segment(r.start_seconds, r.end_seconds, r.text))
+    missing = sum(r is None for r in placed)
+    if missing:
+        print(f"{opt.align_captions}: {missing} of {len(placed)} captions could not be placed and were skipped", file=sys.stderr)
+
+
 def main(argv=None):
     opt = parse(sys.argv[1:] if argv is None else argv)
     if opt.help:
@@ -96,6 +127,15 @@ def main(argv=None):
         print("no audio file specified", file=sys.stderr)
         usage()
         return 1
+    if opt.align_captions is not None:
+        if opt.align is not None:
+            print("--align-captions and --align cannot be combined", file=sys.stderr)
+            return 1
+        if len(opt.audio) != 1:
+            print(f"--align-captions re-times one audio file, got {len(opt.audio)}", file=sys.stderr)
+            return 1
+        run_captions(opt)
+        return None
     transcripts = None
     if opt.align is not None:
         transcripts = read_transcripts(opt.align)

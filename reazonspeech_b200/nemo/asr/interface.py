@@ -78,6 +78,42 @@ class AlignResult(TranscribeResult):
 
 
 @dataclass
+class Caption:
+    """A caption to be found in a recording: the text and the time it was displayed (for a live caption: some seconds after
+    the words were said).  Field names and order follow the reference's oneseg ``Caption`` (pkg/espnet-oneseg/src/interface.py)."""
+    start_seconds: float
+    end_seconds: float
+    text: str
+
+
+@dataclass
+class AlignedCaption:
+    """What ``align_captions`` returns for a caption it placed.  Times are on the recording's own axis: ``start_seconds`` is
+    the time of the frame that emits the caption's first token on the best path, ``end_seconds`` the time of the frame of its
+    last token plus one frame (clipped to the recording).  ``confidence`` is the minimum, over windows of 30 encoder frames
+    (2.4 s), of the mean per-frame log-probability of that path (the plain mean for a shorter span): the analogue of CTC
+    segmentation's ``score_min_mean_over_L``, on this model's scale, not comparable with ESPnet's numbers.
+    ``viterbi_log_prob`` is the best path's log p, ``log_likelihood`` the log p summed over every span and path of the window,
+    ``token_log_probs`` the log p of every token id where the best path emits it.  ``asr`` / ``cer``: the engine's greedy
+    transcript of the placed slice and its character error rate against ``text`` (``with_asr=True``; ``cer`` is None when
+    the normalised caption is empty)."""
+    start_seconds: float
+    end_seconds: float
+    text: str
+    confidence: float
+    viterbi_log_prob: float
+    log_likelihood: float
+    subwords: List[Subword] = field(default_factory=list)
+    token_log_probs: List[float] = field(default_factory=list)
+    asr: Optional[str] = None
+    cer: Optional[float] = None
+
+    @property
+    def duration(self) -> float:
+        return self.end_seconds - self.start_seconds
+
+
+@dataclass
 class TranscribeConfig:
     verbose: bool = True
     raw_hypothesis: bool = False

@@ -82,6 +82,9 @@ class MultiGpuRnntModel:
     def align_tokens(self, waveforms, token_lists, pad: int = 0):
         raise NotImplementedError("the one-process multi-GPU model does not align; load one model per device for align()")
 
+    def align_caption_tokens(self, waveforms, windows, token_lists, pad: int = 0):
+        raise NotImplementedError("the one-process multi-GPU model does not align; load one model per device for align_captions()")
+
     def transcribe(self, audio, batch_size: int = 1, return_hypotheses: bool = True, verbose: bool = True, **_):
         """NeMo's call shape (pkg/nemo-asr/src/transcribe.py:48-53) over all devices."""
         import torch

@@ -10,6 +10,7 @@ transcribe()/decode_hypothesis() therefore run unmodified on it (see INTEGRATION
 from __future__ import annotations
 
 import glob
+import math
 import os
 from dataclasses import dataclass
 from typing import List, Optional, Sequence, Union
@@ -22,10 +23,12 @@ from ...engine import Engine
 from ...tokenizer import PieceTableTokenizer, SentencePieceTokenizer, synthetic_pieces
 from ...weights import load_nemo_archive, random_state_dict
 from .audio import SAMPLERATE, norm_audio, pad_audio
-from .decode import PAD_SECONDS, build_result, decode_hypothesis
-from .interface import AlignResult, AudioData, TranscribeConfig, TranscribeResult
+from .decode import PAD_SECONDS, SECONDS_PER_STEP, build_result, decode_hypothesis
+from .interface import AlignedCaption, AlignResult, AudioData, Caption, TranscribeConfig, TranscribeResult
 
 HF_REPO = "reazon-research/reazonspeech-nemo-v2"
+CAPTION_MARGIN = 25.0          # live captions lag the speech: search from this long before the display time (oneseg's _MARGIN)
+CONFIDENCE_FRAMES = 30         # window of the min-mean caption confidence: 30 encoder frames = 2.4 s
 ENV_CHECKPOINT = "REAZONSPEECH_NEMO_CHECKPOINT"
 ENV_SYNTHETIC = "REAZONSPEECH_B200_SYNTHETIC"
 
@@ -246,6 +249,56 @@ class B200RnntModel:
                 out[i] = (frames[r, :k].tolist(), tok_logp[r, :k].tolist(), float(viterbi[r]), float(loglik[r]))
         return out
 
+    def align_caption_tokens(self, waveforms: Sequence[np.ndarray], windows: Sequence[Sequence[tuple]],
+                             token_lists: Sequence[Sequence[Sequence[int]]], pad: int = 0):
+        """Free-span alignment of known token sequences inside time windows of longer recordings (rs_rnnt_align_spans).
+        ``waveforms``: 16 kHz mono recordings, each encoded ONCE with ``pad`` zero samples on both sides; ``windows[i]``: the
+        (start, end) seconds, on recording i's own axis, of the window each of its captions is searched in; ``token_lists[i]``:
+        the captions' token ids.  -> per recording, per caption ``(lo, frames, token_log_probs, path_logp, viterbi_log_prob,
+        log_likelihood)`` or None (an empty window, or no tokens).  ``lo`` is the window's first encoder frame, ``frames`` the
+        absolute encoder frame of every token on the best path and ``path_logp[t - lo]`` the path's log p at frame t of the
+        window.  Recordings are cut into length-sorted batches as in ``align_tokens``; every batch is one encoder pass and one
+        rs_rnnt_align_spans call over all of its recordings' captions."""
+        eng = self.engine
+        if "alsd.out.w3" not in eng.weights:
+            raise RuntimeError("this model was loaded without the aligner weights: load it with load_model(..., aligner=True)")
+        if not (len(waveforms) == len(windows) == len(token_lists)):
+            raise ValueError(f"align_caption_tokens: {len(waveforms)} waveforms, {len(windows)} window lists, {len(token_lists)} token lists")
+        out: List[List[Optional[tuple]]] = [[None] * len(w) for w in windows]
+        pad_s = pad / SAMPLERATE
+        order = sorted(range(len(waveforms)), key=lambda i: len(waveforms[i]))
+        for lo_b in range(0, len(order), self.max_batch):
+            idx = order[lo_b:lo_b + self.max_batch]
+            wav, lens = self._staging[0].stage([waveforms[i] for i in idx], pad)
+            with torch.cuda.device(eng.device):
+                x = wav.to(eng.device, non_blocking=True)
+                if x.dtype == torch.int16:
+                    x = x.to(torch.float32) * (1.0 / 32768.0)
+                mel, mel_len = eng.log_mel(x, lens.to(eng.device))
+                enc, enc_len = eng.encode(mel, mel_len)
+                T = enc_len.cpu().tolist()
+                items = []                                               # (recording, caption, src, lo, hi, tokens)
+                for r, i in enumerate(idx):
+                    for j, ((start, end), toks) in enumerate(zip(windows[i], token_lists[i])):
+                        lo, hi = window_frames(start, end, T[r], pad_s)
+                        if lo < hi and len(toks) > 0:
+                            items.append((i, j, r, lo, hi, [int(t) for t in toks]))
+                if not items:
+                    continue
+                U = max(len(it[5]) for it in items)
+                spans = torch.tensor([[it[2], it[3], it[4]] for it in items], dtype=torch.int32)
+                targets = torch.zeros(len(items), U, dtype=torch.int32)
+                for k, it in enumerate(items):
+                    targets[k, : len(it[5])] = torch.tensor(it[5], dtype=torch.int32)
+                tgt_len = torch.tensor([len(it[5]) for it in items], dtype=torch.int32)
+                frames, tok_logp, path_logp, viterbi, loglik = [a.cpu() for a in eng.align_spans(
+                    enc, enc_len, spans.to(eng.device), targets.to(eng.device), tgt_len.to(eng.device))]
+            for k, (i, j, _, lo, hi, toks) in enumerate(items):
+                n = len(toks)
+                out[i][j] = (lo, frames[k, :n].tolist(), tok_logp[k, :n].tolist(), path_logp[k, : hi - lo].tolist(),
+                             float(viterbi[k]), float(loglik[k]))
+        return out
+
     def transcribe(self, audio, batch_size: int = 1, return_hypotheses: bool = True, verbose: bool = True, **_):
         waves = [a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a) for a in audio]
         if self.decoding == "alsd":
@@ -403,4 +456,95 @@ def align_batch(model, audios: Sequence[AudioData], texts: Sequence[Union[str, S
         out.append(AlignResult(r.text, r.subwords, r.segments,
                                hypothesis=Hypothesis.from_greedy(tokens, frames, model.cfg.blank) if config.raw_hypothesis else None,
                                log_likelihood=loglik, viterbi_log_prob=viterbi, token_log_probs=tok_logp))
+    return out
+
+
+def window_frames(start: float, end: float, T: int, pad_seconds: float = PAD_SECONDS) -> tuple:
+    """Encoder frames [lo, hi) of the window [start, end] seconds of a recording encoded with ``pad_seconds`` of silence on both
+    sides, clamped to [0, T]: frame f covers [0.08 f - pad, 0.08 (f + 1) - pad) s of the recording, so lo is the frame that
+    holds ``start`` and hi - 1 the frame that holds ``end``.  lo >= hi means an empty window."""
+    lo = math.floor((start + pad_seconds) / SECONDS_PER_STEP)
+    hi = math.floor((end + pad_seconds) / SECONDS_PER_STEP) + 1
+    return min(max(lo, 0), T), min(max(hi, 0), T)
+
+
+def min_mean_confidence(path_logp: Sequence[float], L: int = CONFIDENCE_FRAMES) -> float:
+    """Mean of the per-frame path log-probabilities of a span of n frames when n <= L, else the minimum over its n - L + 1
+    windows of L consecutive frames of their mean (CTC segmentation's ``score_min_mean_over_L``, on this model's scale)."""
+    x = np.asarray(path_logp, np.float64)
+    if len(x) <= L:
+        return float(x.mean())
+    c = np.concatenate(([0.0], np.cumsum(x)))
+    return float(((c[L:] - c[:-L]) / L).min())
+
+
+def add_space(captions: Sequence[AlignedCaption]) -> None:
+    """The oneseg "lax" strategy (pkg/espnet-oneseg/src/align.py:46-51), in place, over consecutive captions in list order:
+    half the gap between two captions, clamped to [0, 3] s, is added to the earlier one's end and taken from the later one's
+    start."""
+    for c0, c1 in zip(captions, captions[1:]):
+        gap = max(min((c1.start_seconds - c0.end_seconds) / 2, 3), 0)
+        c0.end_seconds += gap
+        c1.start_seconds -= gap
+
+
+def align_captions(model, audio: AudioData, captions: Sequence[Caption], *, before: float = CAPTION_MARGIN, after: float = 0.0,
+                   strategy: str = "optim", with_asr: bool = False) -> List[Optional[AlignedCaption]]:
+    """Where in ``audio`` is each caption said: free-span RNN-T alignment of every caption's text inside the window from
+    ``before`` seconds ahead of its start to ``after`` seconds past its end (live captions lag the speech by up to ~25 s),
+    the question ReazonSpeech's corpus builder answers with CTC segmentation (pkg/espnet-oneseg/src/align.py:22-44) and the
+    one that re-timing an SRT / WebVTT file against its audio poses.  The recording is prepared as ``transcribe`` prepares it
+    (norm_audio, 0.5 s of silence on both sides) and encoded once; every caption is placed independently.  Results in input
+    order, None for a caption that could not be placed (an empty window, or text that tokenises to nothing).
+    ``strategy="lax"`` widens consecutive placed captions into half the gap between them (at most 3 s each side), as the
+    reference's "lax" strategy does; ``with_asr=True`` fills ``asr`` and ``cer`` from one greedy ``transcribe_batch`` of the
+    placed slices.  Needs ``load_model(..., aligner=True)``."""
+    return align_captions_batch(model, [audio], [captions], before=before, after=after, strategy=strategy, with_asr=with_asr)[0]
+
+
+def align_captions_batch(model, audios: Sequence[AudioData], caption_lists: Sequence[Sequence[Caption]], *,
+                         before: float = CAPTION_MARGIN, after: float = 0.0, strategy: str = "optim",
+                         with_asr: bool = False) -> List[List[Optional[AlignedCaption]]]:
+    """``align_captions`` for many recordings, cut into length-sorted batches; results in input order."""
+    if strategy not in ("optim", "lax"):
+        raise ValueError(f"strategy must be 'optim' or 'lax', got {strategy!r}")
+    if len(caption_lists) != len(audios):
+        raise ValueError(f"align_captions_batch: {len(audios)} audios but {len(caption_lists)} caption lists")
+    for caps in caption_lists:
+        for c in caps:
+            if c.start_seconds > c.end_seconds:
+                raise ValueError(f"caption {c.text!r} starts at {c.start_seconds} s, after its end {c.end_seconds} s")
+    waves = [np.asarray(norm_audio(a).waveform) for a in audios]
+    ids = [[model.tokenizer.text_to_ids(c.text) for c in caps] for caps in caption_lists]
+    windows = [[(c.start_seconds - before, c.end_seconds + after) for c in caps] for caps in caption_lists]
+    placed = model.align_caption_tokens(waves, windows, ids, pad=int(PAD_SECONDS * SAMPLERATE))
+    out: List[List[Optional[AlignedCaption]]] = []
+    for wave, caps, toks, res in zip(waves, caption_lists, ids, placed):
+        duration = len(wave) / SAMPLERATE
+        row: List[Optional[AlignedCaption]] = []
+        for c, tokens, r in zip(caps, toks, res):
+            if r is None:
+                row.append(None)
+                continue
+            lo, frames, tok_logp, path_logp, viterbi, loglik = r
+            steps = [f + i + 1 for i, f in enumerate(frames)]            # Hypothesis.from_greedy's convention
+            start = min(max(SECONDS_PER_STEP * frames[0] - PAD_SECONDS, 0), duration)
+            end = min(max(SECONDS_PER_STEP * frames[-1] - PAD_SECONDS, 0) + SECONDS_PER_STEP, duration)
+            row.append(AlignedCaption(start, end, c.text, min_mean_confidence(path_logp[frames[0] - lo: frames[-1] - lo + 1]),
+                                      viterbi, loglik, build_result(model.tokenizer, tokens, steps).subwords, tok_logp))
+        out.append(row)
+    if strategy == "lax":
+        for row in out:
+            add_space([r for r in row if r is not None])
+    if with_asr:
+        from ...evaluation.utils import calculate_cer, normalize
+        slices, where = [], []
+        for wave, row in zip(waves, out):
+            for r in row:
+                if r is not None:
+                    slices.append(AudioData(wave[int(r.start_seconds * SAMPLERATE): int(r.end_seconds * SAMPLERATE)], SAMPLERATE))
+                    where.append(r)
+        for r, t in zip(where, transcribe_batch(model, slices) if slices else []):
+            r.asr = t.text
+            r.cer = calculate_cer(r.text, r.asr)["cer"] if normalize(r.text) else None
     return out
